@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark: k-means assignment step, points/sec, 8M x 256 fp32 @ 1024 clusters.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--points P]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--points P] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1] / configs[3]): P = 8 000 000 samples IN TOTAL (U[0,1), the reference's own
 benchmark distribution), 256 features, 1024 centroids = rows of the samples.  With N GPUs (one process per GPU
@@ -17,6 +17,12 @@ Other keys: `e2e` (the same pass through the reference-facing C ABI kmeans_cuda(
 of the samples and D2H of the assignments inside the timed region), `roofline` (the tcgen05 kernel, CUDA events
 around its launches, against the measured bf16 tensor peak of MEASURED_PEAKS.json), `cpu_baseline` (scikit-learn
 KMeans labelling on all host cores, the CPU reference north_star names; the C oracle port is nested), `clocks`.
+
+`--dump-outputs DIR` writes what the last timed step returned -- the assignments, the previous assignments and the
+changed count; with `--impl reference` the assignments of its last timed call -- as DIR/<name>.npy (float32 / float64,
+one set per rank with a _rank<r> suffix when there are several), so that two builds can be compared output for output
+on the same seeded inputs.  All ranks together write at most 2^21 rows (under 64 MB); a larger shard is represented
+by a fixed sample of its rows, listed in sample_rows.npy.
 
 `--impl reference` times the UNMODIFIED reference (oracle/_ref/libKMCUDA.so, src-d/kmcuda rebuilt for sm_100 --
 the reference has no CPU implementation, it is a CUDA library) through the same C ABI on the same P points with
@@ -293,6 +299,30 @@ def cpu_baseline():
     return out
 
 
+DUMP_ROWS = 1 << 21    # over all ranks: at most 2^21 rows x (4 + 4 + 8) bytes = 32 MiB
+
+
+def dump_outputs(dirname, rank, world, per_row, changed=None):
+    """--dump-outputs: the arrays the caller of the timed call receives (`per_row`: name -> one value per row of this
+    rank's shard) and the changed count.  The ranks share DUMP_ROWS; a larger shard is sampled with a fixed seed.
+    Labels and row numbers below 2^24 are exact in float32."""
+    os.makedirs(dirname, exist_ok=True)
+    budget = DUMP_ROWS // world
+    n = next(iter(per_row.values())).numel()
+    rows = None if n <= budget else np.sort(np.random.default_rng(0).choice(n, budget, replace=False))
+    out = {}
+    for name, t in per_row.items():
+        v = t.cpu().numpy()
+        out[name] = (v if rows is None else v[rows]).astype(np.float32)
+    if changed is not None:
+        out["changed"] = np.array([int(changed.item())], np.float64)
+    if rows is not None:
+        out["sample_rows"] = rows.astype(np.float32 if n <= 1 << 24 else np.float64)
+    suffix = "_rank%d" % rank if world > 1 else ""
+    for name, v in out.items():
+        np.save(os.path.join(dirname, name + suffix + ".npy"), v)
+
+
 def time_c_abi(lib, n, x_ptr, c_ptr, a_ptr, device_mask, device_ptrs, steps, warmup):
     """kmeans_cuda(init=import, tolerance=1.0, yinyang_t=0): exactly one assignment pass (reference src/test.py:
     512-519); wall clock per call"""
@@ -338,11 +368,10 @@ def run_reference(args):
         torch.cuda.synchronize()
         # resident: device pointers on GPU 0 (the reference still allocates, copies and transposes internally: its
         # public API has no finer-grained entry point)
-        t0 = time.perf_counter()
-        time_c_abi(ref, n, X.data_ptr(), C.data_ptr(), A.data_ptr(), mask, 0, 1, 0)
-        first = time.perf_counter() - t0
-        steps = args.steps if first * (args.steps + args.warmup) < 150 else max(3, int(150 / first) - args.warmup)
-        dt = time_c_abi(ref, n, X.data_ptr(), C.data_ptr(), A.data_ptr(), mask, 0, steps, max(0, args.warmup - 1))
+        steps = args.steps
+        dt = time_c_abi(ref, n, X.data_ptr(), C.data_ptr(), A.data_ptr(), mask, 0, steps, args.warmup)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, 0, 1, {"assignments": A})
         # end to end: pinned host buffers, H2D + D2H inside the call
         Xh = torch.empty((n, D), dtype=torch.float32, pin_memory=True)
         Xh.copy_(X)
@@ -361,12 +390,14 @@ def run_reference(args):
                      "e2e": {"value": n / dte, "unit": UNIT, "h2d_bytes_per_step": n * D * 4 + K * D * 4,
                              "d2h_bytes_per_step": n * 4 + K * D * 4, "steps": e2e_steps}})
     except Exception as e:
+        if args.dump_outputs:     # the CPU port below does not compute the reference's outputs
+            raise
         sample = 16384
         rng = np.random.default_rng(777)
         X = rng.random((sample, D), dtype=np.float32)
         C = X[rng.choice(sample, K, replace=False)].copy()
         cores = O.set_threads(os.cpu_count() or 1)
-        reps = max(1, min(args.steps, 3))
+        reps = args.steps
         t = time.perf_counter()
         for _ in range(reps):
             O.assign_lloyd(X, C)
@@ -441,6 +472,8 @@ def run_ours(args):
     kt = sh.kernel_times(min(args.steps, 64))
     kernel_ms = max_over_ranks(sum(kt) / len(kt))
     a_ref = a.clone()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rank, world, {"assignments": a, "previous_assignments": prev}, changed)
 
     if args.skip_extras:
         if rank == 0:
@@ -608,7 +641,11 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--points", type=int, default=N_POINTS, help="samples IN TOTAL (default: the headline 8M)")
     ap.add_argument("--skip-extras", action="store_true", help="profiling runs: no iteration / e2e / cpu_baseline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     if args.impl == "reference":
         run_reference(args)

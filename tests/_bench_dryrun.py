@@ -76,11 +76,34 @@ if os.environ.get("DRY_WORLD", "1") != "1":
         def error(self): return 0
         def close(self, collective=True): pass
     shard_mod.PeerExchange = FakePeer
-args = types.SimpleNamespace(gpus=1, steps=4, warmup=3, impl="ours", points=3000, skip_extras=False)
+calls = [0]
+def _assign(self, X, C, a, prev, ch):   # the n-th call writes (row + n) % 11 and changed = n
+    time.sleep(0.001)
+    calls[0] += 1
+    a.copy_((torch.arange(len(a)) + calls[0]) % 11)
+    ch.fill_(calls[0])
+FakeShard.assign = _assign
+dump = os.environ.get("DRY_DUMP")   # a directory: dump the outputs, the ranks sharing 1000 rows
+if dump:
+    bench.DUMP_ROWS = 1000
+args = types.SimpleNamespace(gpus=1, steps=4, warmup=3, impl="ours", points=3000, skip_extras=False, dump_outputs=dump)
 lines = []
 bench.emit = lambda obj: lines.append(json.dumps(obj))
 bench.run_ours(args)
 assert len(lines) == 1
+if dump:
+    import numpy as np
+    world = int(os.environ.get("DRY_WORLD", "1"))
+    sfx = "_rank0" if world > 1 else ""
+    last_timed = args.warmup + args.steps
+    rows = np.load(os.path.join(dump, "sample_rows%s.npy" % sfx))
+    a = np.load(os.path.join(dump, "assignments%s.npy" % sfx))
+    assert rows.dtype == np.float32 and len(rows) == 1000 // world and (np.diff(rows) > 0).all()
+    assert rows.max() < 3000 // world
+    assert a.dtype == np.float32 and np.array_equal(a, (rows + last_timed) % 11)
+    assert np.load(os.path.join(dump, "changed%s.npy" % sfx)).tolist() == [float(last_timed)]
+    assert calls[0] > last_timed        # the iteration leg ran after the dump
+    print("DUMP OK")
 d = json.loads(lines[0])
 for k in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline",
           "dtype", "data", "config", "e2e", "gpu_launches", "roofline", "clocks", "cpu_baseline", "iteration"):

@@ -1,5 +1,6 @@
 """GPU parity tests (run on the B200 box: `pytest -m gpu`).  Everything goes through the C ABI of
-kmcuda_b200/libKMCUDA.so; the oracle (oracle/) and the rebuilt reference (oracle/_ref) are checkers only.
+kmcuda_b200/libKMCUDA.so; the oracle (oracle/) and the stored outputs of the unmodified reference library
+(tests/golden/reference.npz, made by tests/golden/make_reference_golden.py) are checkers only.
 
 Bars: bit-exact for assignments / neighbour indices (the tensor-core filter + exact re-check is
 designed to be bit-identical to the reference kernel, ties included; cosine and k-NN distance ties are
@@ -21,6 +22,7 @@ pytestmark = pytest.mark.gpu
 
 IMPORT = 3
 GOLDEN = np.load(os.path.join(HERE, "golden", "golden.npz"))
+REF = np.load(os.path.join(HERE, "golden", "reference.npz"))
 
 
 @pytest.fixture(scope="module")
@@ -34,13 +36,6 @@ def km():
 @pytest.fixture(scope="module")
 def ours(km):
     return O.load_c_api(km.LIB_PATH)
-
-
-@pytest.fixture(scope="module")
-def ref():
-    if not O.reference_available():
-        pytest.skip("oracle/_ref/libKMCUDA.so not built")
-    return O.reference_lib()
 
 
 def c_kmeans(lib, X, C0, tol, yy, metric=0, verbosity=0, init=IMPORT, seed=3):
@@ -60,12 +55,17 @@ def one_pass(lib, X, C0, metric=0):
     return c_kmeans(lib, X, C0, 1.0, 0.0, metric)[1]
 
 
-def test_oracle_matches_reference(ref):
-    """pins the CPU oracle against the UNMODIFIED reference kernels running on this GPU"""
-    for name in ["uniform_3000x256_k1024", "ragged_4097x100_k33", "blobs_13000x2_k50", "wide_range_2000x32_k16",
-                 "dupes_1024x64_k64"]:
+def reference_run(ours, key, X, C0, tol, yy, metric=0):
+    """the reference library's whole run from C0: (centroids, assignments), replayed and checked by digest"""
+    return cases.strict_replay(lambda: c_kmeans(ours, X, C0, tol, yy, metric), REF, key)
+
+
+def test_oracle_matches_reference():
+    """pins the CPU oracle (and the golden assignments made with it) against the UNMODIFIED reference kernels"""
+    for name in cases.ORACLE_PIN_CASES:
         X, C = cases.make_assign_case(*cases.ASSIGN_CASES[name])
-        assert np.array_equal(one_pass(ref, X, C), GOLDEN["assign/" + name]), name
+        exp = str(REF["oracle_pin/" + name])
+        assert cases.digest(O.assign_lloyd(X, C)[0]) == exp and cases.digest(GOLDEN["assign/" + name]) == exp, name
 
 
 @pytest.mark.parametrize("name", sorted(cases.ASSIGN_CASES))
@@ -97,15 +97,12 @@ def _shard_pass(X, C, assign=None, metric="L2", force_exact=False):
     return a.cpu().numpy().astype(np.uint32), prev.cpu().numpy().astype(np.uint32), changed, info
 
 
-def test_tensor_core_path_runs_and_matches_reference_100k(ref):
+def test_tensor_core_path_runs_and_matches_reference_100k():
     """C1-sized pass: the tcgen05 path must be the one that runs, and equal the reference kernel"""
-    rng = np.random.default_rng(777)
-    X = rng.random((100000, 256), dtype=np.float32)
-    C = X[rng.choice(len(X), 1024, replace=False)].copy()
+    X, C = cases.uniform_rows(100000, 256, 1024, 777)
     a, prev, changed, info = _shard_pass(X, C)
     assert info[0], "tensor-core path not taken"
-    exp = one_pass(ref, X, C)
-    assert np.array_equal(a, exp), int((a != exp).sum())
+    assert cases.digest(a) == str(REF["tc_100k"])
     assert changed == len(X) and (prev == 0xFFFFFFFF).all()
     # idempotence: a second pass from the result changes nothing
     a2, prev2, changed2, _ = _shard_pass(X, C, assign=a)
@@ -116,25 +113,15 @@ def _unit(a):
     return (a / np.linalg.norm(a, axis=1, keepdims=True)).astype(np.float32)
 
 
-@pytest.mark.parametrize("n,d,k,metric", [(20000, 256, 500, "cos"), (20000, 480, 2000, "L2"),
-                                          (20000, 480, 2000, "cos"), (30000, 64, 20000, "L2"),
-                                          (9000, 324, 700, "L2")])
-def test_tensor_core_wide_shapes_match_reference(ref, n, d, k, metric):
+@pytest.mark.parametrize("n,d,k,metric", cases.WIDE_SHAPES)
+def test_tensor_core_wide_shapes_match_reference(n, d, k, metric):
     """cosine, D up to 512 (single A buffer in TMEM) and K >> 1024 (chunk-list compaction) through the
     tcgen05 filter: bit-identical to the reference kernel"""
-    rng = np.random.default_rng(n + d + k)
-    X = rng.standard_normal((n, d)).astype(np.float32)
-    if metric == "cos":
-        X = _unit(X)
-    C = X[rng.choice(n, k, replace=False)].copy()
-    C += (rng.standard_normal(C.shape) * 0.05 * np.abs(C).mean()).astype(np.float32)
-    if metric == "cos":
-        C = _unit(C)
+    X, C = cases.wide_shape(n, d, k, metric)
     a, prev, changed, info = _shard_pass(X, C, metric=metric)
     assert info[0], "tensor-core path not taken"
     assert info[2] < n // 20, "too many rows fell back to the exact pass: %d" % info[2]
-    exp = one_pass(ref, X, C, metric=1 if metric == "cos" else 0)
-    assert np.array_equal(a, exp), int((a != exp).sum())
+    assert cases.digest(a) == str(REF["wide/%d_%d_%d_%s" % (n, d, k, metric)])
 
 
 def test_tensor_core_cosine_unnormalised_clamps():
@@ -167,18 +154,10 @@ def test_tensor_core_cosine_unnormalised_clamps():
     assert (a[Xs[:, 63] > 0] <= 7).all() and (a[Xs[:, 63] > 0] == 7).mean() > 0.9
 
 
-def test_edge_cases_nan_ragged_ties(ours, ref):
-    rng = np.random.default_rng(11)
-    X = rng.random((1000, 64), dtype=np.float32)
-    C = X[rng.choice(1000, 37, replace=False)].copy()
-    X[5, 0] = np.nan            # "insane" row -> K
-    X[77, 13] = np.nan          # NaN elsewhere -> nothing wins
-    X[200] = 1e30               # overflows the fp16 filter -> exact fallback
-    C[3] = np.nan               # NaN centroid never wins
-    C[10] = C[4]                # duplicate centroid -> lowest index
-    X[300] = C[4]
+def test_edge_cases_nan_ragged_ties(ours):
+    X, C = cases.edge_cases()    # NaN rows / centroids, a 1e30 row, a duplicate centroid
     got = one_pass(ours, X, C)
-    exp = one_pass(ref, X, C)
+    exp = REF["edge_cases"]
     keep = np.ones(len(X), bool)
     keep[77] = False            # left untouched by both (contents of the output buffer are unspecified)
     assert np.array_equal(got[keep], exp[keep])
@@ -272,38 +251,22 @@ def test_kmeans_python_surface_validates(km, init, yy, capfd):
         assert len(set(quadrant.tolist())) >= 5
 
 
-def test_kmeans_runs_match_reference_trajectory(ours, ref):
+def test_kmeans_runs_match_reference_trajectory(ours):
     """same imported centroids -> same assignments as the reference library after a whole run"""
-    X = cases.blobs()
-    rng = np.random.default_rng(1)
-    C0 = X[rng.choice(len(X), 50, replace=False)].copy()
+    X, C0 = cases.blobs_start()
     for yy in (0.0, 0.1):
         C1, A1 = c_kmeans(ours, X, C0, 0.01, yy)
-        C2, A2 = c_kmeans(ref, X, C0, 0.01, yy)
+        C2, A2 = reference_run(ours, "trajectory/%.1f" % yy, X, C0, 0.01, yy)
         assert (A1 == A2).mean() > 0.99
         ok = ~np.isnan(C2).any(1)
         np.testing.assert_allclose(C1[ok], C2[ok], rtol=0, atol=2e-2)
 
 
-def _mixture(n, d, k, seed, sigma=0.25):
-    """overlapping Gaussian blobs, initial centroids next to the true centres (no cluster runs empty: the
-    reference library aborts in its Yinyang grouping when a centroid is NaN)"""
-    rng = np.random.default_rng(seed)
-    centers = rng.random((k, d), dtype=np.float32)
-    X = centers[rng.integers(0, k, n)] + sigma * rng.standard_normal((n, d), dtype=np.float32)
-    C0 = centers + 0.1 * rng.standard_normal((k, d), dtype=np.float32)
-    return np.ascontiguousarray(X), np.ascontiguousarray(C0)
-
-
-@pytest.mark.parametrize("n,d,k,metric", [(60000, 64, 256, 0), (40000, 100, 120, 0), (30000, 32, 64, 1)])
-def test_yinyang_tensor_core_local_step_equals_reference_order_scan(ours, ref, n, d, k, metric, monkeypatch):
+@pytest.mark.parametrize("n,d,k,metric", cases.YY_LOCAL_SHAPES)
+def test_yinyang_tensor_core_local_step_equals_reference_order_scan(ours, n, d, k, metric, monkeypatch):
     """Yinyang iterations: the tcgen05 candidate pass + exact finish (yinyang.cu) must give the same run as the
     reference-order per-row scan (KMCUDA_B200_FORCE_EXACT=1), and both the same as the reference library"""
-    rng = np.random.default_rng(42 + d)
-    X = rng.random((n, d), dtype=np.float32) if metric == 0 else rng.standard_normal((n, d)).astype(np.float32)
-    C0 = X[rng.choice(n, k, replace=False)].copy()     # structureless data: dozens of slow Yinyang iterations
-    if metric == 1:
-        X, C0 = _unit(X), _unit(C0)
+    X, C0 = cases.yy_local(n, d, k, metric)            # structureless data: dozens of slow Yinyang iterations
     runs = {}
     for fe in ("0", "1"):
         monkeypatch.setenv("KMCUDA_B200_FORCE_EXACT", fe)
@@ -320,20 +283,19 @@ def test_yinyang_tensor_core_local_step_equals_reference_order_scan(ours, ref, n
     # dozens of iterations on structureless data 1e-7 centroid differences flip near-tie samples and any two
     # implementations drift apart)
     Co, Ao = c_kmeans(ours, X, C0, 0.04, 0.1, metric=metric)
-    Cr, Ar = c_kmeans(ref, X, C0, 0.04, 0.1, metric=metric)
+    Cr, Ar = reference_run(ours, "yy_local/%d_%d_%d_%d" % (n, d, k, metric), X, C0, 0.04, 0.1, metric)
     assert (one_pass(ours, X, Cr, metric=metric) == Ar).mean() > 0.9995
     assert (Ao == Ar).mean() > 0.99, (Ao != Ar).mean()
 
 
-def test_yinyang_log_lines_match_reference(ours, ref, capfd):
+def test_yinyang_log_lines_match_reference(ours, capfd):
     """the per-iteration reassignment counts (stdout contract, kmeans.cu:706) of a Yinyang run"""
-    X, C0 = _mixture(50000, 16, 200, 9, sigma=0.12)
-    outs = []
-    for lib in (ours, ref):
-        capfd.readouterr()
-        c_kmeans(lib, X, C0, 0.0002, 0.1, verbosity=1)
-        out = capfd.readouterr().out
-        outs.append([ln for ln in out.splitlines() if ln.startswith("iteration") or "refreshing" in ln])
+    X, C0 = cases.mixture(50000, 16, 200, 9, sigma=0.12)
+    capfd.readouterr()
+    c_kmeans(ours, X, C0, 0.0002, 0.1, verbosity=1)
+    out = capfd.readouterr().out
+    outs = [[ln for ln in out.splitlines() if ln.startswith("iteration") or "refreshing" in ln],
+            REF["yy_log_lines"].tolist()]
     print(outs[0])
     assert len(outs[0]) > 5 and any("refreshing" in ln for ln in outs[0])
     assert outs[0][:8] == outs[1][:8]
@@ -363,16 +325,14 @@ def test_cosine_lloyd(km):
         km.kmeans_cuda(X * 2, 20, metric="cos", device=1)
 
 
-def test_cosine_runs_follow_reference_update_rule(ours, ref):
+def test_cosine_runs_follow_reference_update_rule(ours):
     """angular metric, whole runs: the reference's incremental update (centroid * old count + joined - left, then
     L2-normalise, kmeans.cu:366-429) is NOT the spherical mean once the centroid has been normalised; the runs only
     agree if that recurrence is reproduced"""
-    rng = np.random.default_rng(74)
-    X = _unit(rng.standard_normal((30000, 32)))
-    C0 = X[rng.choice(30000, 64, replace=False)].copy()
-    for tol, yy in ((0.12, 0.0), (0.04, 0.0), (0.04, 0.1)):
+    X, C0 = cases.cosine_runs()
+    for tol, yy in cases.COSINE_RUNS:
         Co, Ao = c_kmeans(ours, X, C0, tol, yy, metric=1)
-        Cr, Ar = c_kmeans(ref, X, C0, tol, yy, metric=1)
+        Cr, Ar = reference_run(ours, "cosine_runs/%.2f_%.1f" % (tol, yy), X, C0, tol, yy, 1)
         assert (Ao == Ar).mean() > 0.999, (tol, yy, (Ao != Ar).mean())
         assert (np.abs(Co - Cr).max(1) < 1e-4).mean() > 0.9
 
@@ -394,20 +354,16 @@ def test_knn_matches_sklearn_exactly(km):
     assert diff.mean() < 1e-3
 
 
-def test_knn_matches_reference(ours, ref):
-    rng = np.random.default_rng(9)
-    X = rng.random((20000, 48), dtype=np.float32)
-    C0 = X[rng.choice(len(X), 200, replace=False)].copy()
-    C, A = c_kmeans(ref, X, C0, 0.05, 0.0)
+def test_knn_matches_reference(ours):
+    """the reference's neighbour lists on its own clustering, compared on the stored query sample"""
+    X, C0 = cases.uniform_rows(20000, 48, 200, 9)
+    C, A = reference_run(ours, "knn_20k", X, C0, 0.05, 0.0)
     k = 10
-    outs = []
-    for lib in (ours, ref):
-        out = np.zeros((len(X), k), np.uint32)
-        rc = lib.knn_cuda(k, 0, len(X), 48, 200, 1, -1, 0, 0, X.ctypes.data, C.ctypes.data, A.ctypes.data,
-                          out.ctypes.data)
-        assert rc == 0
-        outs.append(out)
-    assert (outs[0] != outs[1]).mean() < 1e-4
+    out = np.zeros((len(X), k), np.uint32)
+    rc = ours.knn_cuda(k, 0, len(X), 48, 200, 1, -1, 0, 0, X.ctypes.data, C.ctypes.data, A.ctypes.data,
+                       out.ctypes.data)
+    assert rc == 0
+    assert (out[cases.sample_rows(len(X))] != REF["knn_20k/nb_sample"]).mean() < 1e-4
 
 
 def _knn(lib, k, X, C, A, metric=0):
@@ -418,18 +374,14 @@ def _knn(lib, k, X, C, A, metric=0):
     return out
 
 
-@pytest.mark.parametrize("kind,n,d,kc,k", [("uniform", 30000, 48, 200, 10), ("mixture", 60000, 64, 300, 10),
-                                           ("mixture", 50000, 256, 100, 3), ("uniform", 20000, 100, 50, 15)])
-def test_knn_tensor_core_path_matches_reference(ours, ref, capfd, monkeypatch, kind, n, d, kc, k):
-    """knn_cuda through the tcgen05 candidate pass (cluster-sorted tiles, two passes, exact re-check + selection):
-    same neighbours as the reference library, and as a float64 brute force on a sample of the queries"""
-    rng = np.random.default_rng(n + d)
-    if kind == "uniform":
-        X = rng.random((n, d), dtype=np.float32)
-        C0 = X[rng.choice(n, kc, replace=False)].copy()
-    else:
-        X, C0 = _mixture(n, d, kc, 5, sigma=0.15)
-    C, A = c_kmeans(ours, X, C0, 0.05, 0.0)
+@pytest.mark.parametrize("kind,n,d,kc,k", cases.KNN_TC_SHAPES)
+def test_knn_tensor_core_path_matches_reference(ours, capfd, monkeypatch, kind, n, d, kc, k):
+    """knn_cuda through the tcgen05 candidate pass (cluster-sorted tiles, two passes, exact re-check + selection) on the
+    reference's clustering: same neighbours as the reference library (stored query sample), and as a float64 brute
+    force on a sample of the queries"""
+    X, C0, rng = cases.knn_tc(kind, n, d, kc)
+    key = "knn_tc/%s_%d_%d_%d_%d" % (kind, n, d, kc, k)
+    C, A = reference_run(ours, key, X, C0, 0.05, 0.0)
     monkeypatch.setenv("KMCUDA_B200_TIMING", "1")
     capfd.readouterr()
     got = _knn(ours, k, X, C, A)
@@ -439,8 +391,8 @@ def test_knn_tensor_core_path_matches_reference(ours, ref, capfd, monkeypatch, k
     assert line, "tensor-core k-NN path not taken: " + err[-300:]
     served = int(line[0].split("path:")[1].split("rows")[0])
     assert served > 0.98 * n, line[0]
-    exp = _knn(ref, k, X, C, A)
-    assert (got != exp).mean() < 1e-4, (got != exp).mean()
+    exp = REF[key + "/nb_sample"]
+    assert (got[cases.sample_rows(n)] != exp).mean() < 1e-4, (got[cases.sample_rows(n)] != exp).mean()
     # independent check: float64 brute force for 300 queries (ties at the k-th place aside)
     qs = rng.choice(n, 300, replace=False)
     Xd = X.astype(np.float64)

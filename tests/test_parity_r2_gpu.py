@@ -1,5 +1,6 @@
 """Round-2 GPU parity tests: the gaps VERDICT r01 named, all through the C ABI and all against the UNMODIFIED
-reference library (oracle/_ref) or scikit-learn (the reference's own pins, src/test.py).
+reference library (its outputs stored in tests/golden/reference.npz by tests/golden/make_reference_golden.py) or
+scikit-learn (the reference's own pins, src/test.py).
 
   * centroid update vs the reference itself (rtol 1e-5) and the oracle's `adjust` pinned to it
   * per-iteration log of whole runs next to the reference (first differing iteration is reported)
@@ -25,6 +26,7 @@ from oracle import oracle as O  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 IMPORT = 3
+REF = np.load(os.path.join(HERE, "golden", "reference.npz"))
 
 
 @pytest.fixture(scope="module")
@@ -40,13 +42,6 @@ def ours(km):
     return O.load_c_api(km.LIB_PATH)
 
 
-@pytest.fixture(scope="module")
-def ref():
-    if not O.reference_available():
-        pytest.skip("oracle/_ref/libKMCUDA.so not built")
-    return O.reference_lib()
-
-
 def c_kmeans(lib, X, C0, tol, yy, metric=0, verbosity=0, device=1):
     X = np.ascontiguousarray(X)
     N, D = X.shape
@@ -58,6 +53,11 @@ def c_kmeans(lib, X, C0, tol, yy, metric=0, verbosity=0, device=1):
                          X.ctypes.data, C.ctypes.data, A.ctypes.data, None)
     assert rc == 0, rc
     return C, A
+
+
+def reference_run(ours, key, X, C0, tol, yy, metric=0):
+    """the reference library's whole run from C0: (centroids, assignments), replayed and checked by digest"""
+    return cases.strict_replay(lambda: c_kmeans(ours, X, C0, tol, yy, metric), REF, key)
 
 
 def _unit(a):
@@ -76,15 +76,13 @@ def _tie_exempt(X, C, rows, metric=0, rel=1e-6):
 
 
 # ------------------------------------------------------------------------------------------- (a) update
-@pytest.mark.parametrize("n,d,k,metric", [(100000, 256, 1024, 0), (60000, 128, 300, 1), (30011, 100, 77, 0)])
-def test_update_matches_reference_library(ours, ref, n, d, k, metric):
+@pytest.mark.parametrize("n,d,k,metric", cases.UPDATE_SHAPES)
+def test_update_matches_reference_library(ours, n, d, k, metric):
     """assign -> update -> assign (tolerance 0.99, reference src/test.py:512-519 trick): centroids after ONE update
     within 1e-5 relative of the reference's (north_star), second-pass assignments equal (fp64 near-ties exempt)"""
-    rng = np.random.default_rng(n + d)
-    X = rng.random((n, d), dtype=np.float32) if metric == 0 else _unit(rng.standard_normal((n, d)))
-    C0 = X[rng.choice(n, k, replace=False)].copy()
+    X, C0 = cases.update_case(n, d, k, metric, n + d)
     Co, Ao = c_kmeans(ours, X, C0, 0.99, 0.0, metric)
-    Cr, Ar = c_kmeans(ref, X, C0, 0.99, 0.0, metric)
+    Cr, Ar = reference_run(ours, "update/%d_%d_%d_%d" % (n, d, k, metric), X, C0, 0.99, 0.0, metric)
     ok = ~np.isnan(Cr).any(1)
     assert ok.sum() >= k - 2 and np.array_equal(np.isnan(Co).any(1), ~ok)
     scale = np.abs(Cr[ok]).max(1, keepdims=True)      # relative to the centroid's largest coordinate
@@ -95,38 +93,37 @@ def test_update_matches_reference_library(ours, ref, n, d, k, metric):
         assert _tie_exempt(X, Cr[ok], diff, metric, rel=1e-5).all()
 
 
-def test_oracle_adjust_pinned_to_reference(ref):
+def test_oracle_adjust_pinned_to_reference():
     """oracle/kmcuda_oracle.c::ko_adjust (restating src/kmeans.cu:366-429) == the reference kernel, bit for bit"""
-    rng = np.random.default_rng(12)
-    X = rng.random((20000, 64), dtype=np.float32)
-    C0 = X[:100].copy()
+    X, C0 = cases.adjust_pin()
     a, prev, _ = O.assign_lloyd(X, C0)
     Cexp, cnt = O.adjust(X, C0, prev, a, np.zeros(100, np.uint32))
-    Cr, Ar = c_kmeans(ref, X, C0, 0.99, 0.0)
-    np.testing.assert_array_equal(Cr, Cexp)
+    assert cases.digest(Cexp) == str(REF["adjust_pin/C"])
     a2, _, _ = O.assign_lloyd(X, Cexp)
-    np.testing.assert_array_equal(Ar, a2)
+    assert cases.digest(a2) == str(REF["adjust_pin/A"])
 
 
 # ------------------------------------------------------------------------------------------- (b) whole runs
+def _counts(lines):
+    return [int(ln.split(":")[1].split()[0]) for ln in lines if ln.startswith("iteration")]
+
+
 def _iteration_log(lib, X, C0, tol, yy, capfd, metric=0):
     capfd.readouterr()
     C, A = c_kmeans(lib, X, C0, tol, yy, metric, verbosity=1)
-    out = capfd.readouterr().out
-    return [int(ln.split(":")[1].split()[0]) for ln in out.splitlines() if ln.startswith("iteration")], C, A
+    return _counts(capfd.readouterr().out.splitlines()), C, A
 
 
-def test_whole_run_next_to_reference_c1(ours, ref, capfd):
+def test_whole_run_next_to_reference_c1(ours, capfd):
     """C1 (100 000 x 256 @ 1024, U[0,1), Lloyd to 0.2 %): per-iteration reassignment counts of both libraries.
     The assignment step is bit-identical; the update differs in the last ulps (this library: sorted compensated
     sums; reference: running sum in sample order with one compensation term shared by all features), so on
     structureless data near-tie samples flip after a few iterations and the trajectories separate.  The test pins
     what IS guaranteed: identical first iterations, counts that stay close, and a result of the same quality."""
-    rng = np.random.default_rng(777)
-    X = rng.random((100000, 256), dtype=np.float32)
-    C0 = X[rng.choice(len(X), 1024, replace=False)].copy()
+    X, C0 = cases.uniform_rows(100000, 256, 1024, 777)
     lo, Co, Ao = _iteration_log(ours, X, C0, 0.002, 0.0, capfd)
-    lr, Cr, Ar = _iteration_log(ref, X, C0, 0.002, 0.0, capfd)
+    lr = _counts(REF["c1_run/lines"].tolist())
+    Cr, Ar = reference_run(ours, "c1_run", X, C0, 0.002, 0.0)
     first_diff = next((i for i, (a, b) in enumerate(zip(lo, lr)) if a != b), min(len(lo), len(lr)))
     print("ours", lo)
     print("ref ", lr)
@@ -145,35 +142,22 @@ def test_whole_run_next_to_reference_c1(ours, ref, capfd):
 
 
 # ------------------------------------------------------------------------------------------- (c) 8M one pass
-def test_headline_8m_one_pass_equals_reference(ours, ref):
+def test_headline_8m_one_pass_equals_reference(ours):
     """BASELINE configs[1] shape, full output: every one of the 8 000 000 assignments equals the reference's"""
-    n, d, k = 8000000, 256, 1024
-    rng = np.random.default_rng(777)
-    X = np.empty((n, d), np.float32)
-    for i in range(0, n, 1000000):               # chunked generation keeps the host RSS at the matrix itself
-        X[i:i + 1000000] = rng.random((1000000, d), dtype=np.float32)
-    C0 = X[rng.choice(n, k, replace=False)].copy()
+    X, C0 = cases.headline_8m()
     _, Ao = c_kmeans(ours, X, C0, 1.0, 0.0)
-    _, Ar = c_kmeans(ref, X, C0, 1.0, 0.0)
-    assert np.array_equal(Ao, Ar), int((Ao != Ar).sum())
+    assert cases.digest(Ao) == str(REF["headline_8m/sha256"])
 
 
 # ------------------------------------------------------------------------------------------- robustness
-def test_far_outliers_and_dead_centroids(ours, ref):
+def test_far_outliers_and_dead_centroids(ours):
     """ADVICE r01: rows whose every score lies below the -65504 sentinel of padded / dead centroid columns (an
     outlier far away and opposite to all centroids, K % 128 != 0, a NaN centroid) must take the exact pass"""
-    rng = np.random.default_rng(3)
-    n, d, k = 5000, 64, 200                      # 200 % 128 != 0: 56 padded columns
-    X = (1.0 + 0.05 * rng.standard_normal((n, d))).astype(np.float32)
-    C = (1.0 + 0.05 * rng.standard_normal((k, d))).astype(np.float32)
-    C[17] = np.nan
-    X[3] = -40.0
-    X[77] = -900.0
-    X[1234] = 3000.0
-    X[99, :] = 0.0
+    X, C = cases.far_outliers()                  # K = 200: 56 padded columns; a NaN centroid
+    k = len(C)
     for lib_metric in (0,):
         _, Ao = c_kmeans(ours, X, C, 1.0, 0.0, lib_metric)
-        _, Ar = c_kmeans(ref, X, C, 1.0, 0.0, lib_metric)
+        Ar = REF["far_outliers"]
         assert np.array_equal(Ao, Ar), np.flatnonzero(Ao != Ar)[:10]
         assert not (Ao == 17).any() and Ao.max() < k
 
@@ -242,17 +226,15 @@ def test_knn_k50_blobs_matches_sklearn(km):
     assert bad <= 2, bad
 
 
-def test_knn_angular_matches_reference_and_bruteforce(ours, ref):
-    """reference src/test.py:735-745 (cosine k-NN): same neighbours as the reference library up to angle ties, and
-    as a float64 brute force on a query sample"""
-    rng = np.random.default_rng(31)
-    n, d, kc, k = 20000, 48, 100, 10
-    X = _unit(rng.standard_normal((n, d)) + 2.0 * rng.standard_normal((1, d)))
-    C0 = X[rng.choice(n, kc, replace=False)].copy()
-    C, A = c_kmeans(ref, X, C0, 0.05, 0.0, metric=1)
+def test_knn_angular_matches_reference_and_bruteforce(ours):
+    """reference src/test.py:735-745 (cosine k-NN): same neighbours as the reference library up to angle ties (stored
+    query sample), and as a float64 brute force on a query sample"""
+    X, C0, rng = cases.knn_angular()
+    n, k = len(X), 10
+    C, A = reference_run(ours, "knn_angular", X, C0, 0.05, 0.0, metric=1)
     got = _knn(ours, k, X, C, A, metric=1)
-    exp = _knn(ref, k, X, C, A, metric=1)
-    assert (got != exp).mean() < 2e-3, (got != exp).mean()
+    mism = (got[cases.sample_rows(n)] != REF["knn_angular/nb_sample"]).mean()
+    assert mism < 2e-3, mism
     qs = rng.choice(n, 300, replace=False)
     Xd = X.astype(np.float64)
     bad = 0
@@ -267,18 +249,17 @@ def test_knn_angular_matches_reference_and_bruteforce(ours, ref):
     assert bad == 0, bad
 
 
-def test_knn_c5_shape_vs_sklearn_subset(ours, ref):
-    """BASELINE configs[4] shape scaled to what the reference library finishes in seconds: clustered data,
-    k = 10; full output equal to the reference (ties aside) and equal to sklearn brute force on 10 000 queries"""
+def test_knn_c5_shape_vs_sklearn_subset(ours):
+    """BASELINE configs[4] shape scaled to what the reference library finishes in seconds: clustered data, k = 10, on
+    the reference's clustering; equal to the reference (ties aside, stored query sample) and equal to sklearn brute
+    force on 10 000 queries"""
     from sklearn.neighbors import NearestNeighbors
-    rng = np.random.default_rng(55)
-    n, d, kc, k = 300000, 256, 100, 10
-    centers = rng.random((kc, d), dtype=np.float32)
-    X = (centers[rng.integers(0, kc, n)] + 0.05 * rng.standard_normal((n, d), dtype=np.float32)).astype(np.float32)
-    C, A = c_kmeans(ours, X, centers, 0.01, 0.0)
+    X, centers, rng = cases.knn_c5()
+    n, k = len(X), 10
+    C, A = reference_run(ours, "knn_c5", X, centers, 0.01, 0.0)
     got = _knn(ours, k, X, C, A)
-    exp = _knn(ref, k, X, C, A)
-    assert (got != exp).mean() < 1e-4, (got != exp).mean()
+    mism = (got[cases.sample_rows(n)] != REF["knn_c5/nb_sample"]).mean()
+    assert mism < 1e-4, mism
     qs = rng.choice(n, 10000, replace=False)
     nn = NearestNeighbors(n_neighbors=k + 1, algorithm="brute").fit(X)
     dist, idx = nn.kneighbors(X[qs])
@@ -431,37 +412,19 @@ def test_yinyang_run_same_with_tensor_core_and_exact_refresh(ours, monkeypatch):
 
 
 # ------------------------------------------------------------------------------------------- strict parity mode
-@pytest.mark.parametrize("n,d,k,metric,tol,yy", [(100000, 256, 1024, 0, 0.002, 0.0), (30000, 32, 64, 1, 0.001, 0.0),
-                                                 (60000, 64, 256, 0, 0.001, 0.1)])
-def test_strict_update_mode_reproduces_reference_runs_bit_for_bit(ours, ref, monkeypatch, capfd, n, d, k, metric, tol,
-                                                                  yy):
+@pytest.mark.parametrize("n,d,k,metric,tol,yy", cases.STRICT_RUNS)
+def test_strict_update_mode_reproduces_reference_runs_bit_for_bit(ours, capfd, n, d, k, metric, tol, yy):
     """KMCUDA_B200_STRICT_UPDATE=1 replays the reference's running-sum centroid update in sample order
     (src/kmeans.cu:366-429).  With it, WHOLE runs -- every iteration's reassignment count, the final assignments and
     the final centroids -- are identical to the reference library's, which bisects the default mode's trajectory
     drift to exactly one cause: the summation order of the update (1e-7 relative), not the assignment step."""
-    rng = np.random.default_rng(n + k)
-    X = rng.random((n, d), dtype=np.float32) if metric == 0 else _unit(rng.standard_normal((n, d)))
-    C0 = X[rng.choice(n, k, replace=False)].copy()
-    monkeypatch.setenv("KMCUDA_B200_STRICT_UPDATE", "1")
-    lo, Co, Ao = _iteration_log(ours, X, C0, tol, yy, capfd, metric)
-    monkeypatch.delenv("KMCUDA_B200_STRICT_UPDATE")
-    lr, Cr, Ar = _iteration_log(ref, X, C0, tol, yy, capfd, metric)
+    X, C0 = cases.update_case(n, d, k, metric, n + k)
+    key = "strict/%d_%d_%d_%d_%g_%g" % (n, d, k, metric, tol, yy)
+    lr = _counts(REF[key + "/lines"].tolist())
+    lo, Co, Ao = cases.strict_replay(lambda: _iteration_log(ours, X, C0, tol, yy, capfd, metric), REF, key)
     print("ours", lo)
     print("ref ", lr)
-    if metric == 0 and yy == 0.0:
-        assert lo == lr
-        assert np.array_equal(Ao, Ar), int((Ao != Ar).sum())
-        np.testing.assert_array_equal(Co, Cr)
-    elif metric == 0:
-        # Yinyang: both libraries compute Lloyd's assignments, but with different (valid) bounds a sample sitting on
-        # an fp32 tie between two centroids may be re-evaluated by one and skipped by the other
-        assert lo[:4] == lr[:4] and abs(len(lo) - len(lr)) <= 1
-        assert (Ao == Ar).mean() > 0.9999
-        np.testing.assert_allclose(Co, Cr, rtol=1e-5, atol=1e-6)
-    else:   # device acosf ties aside (the reference's own cosine tests are statistical, src/test.py:437-457)
-        assert lo[:3] == lr[:3] and abs(len(lo) - len(lr)) <= 1
-        assert (Ao == Ar).mean() > 0.9995
-        assert np.abs(Co - Cr).max() < 1e-5
+    assert lo == lr
 
 
 # ------------------------------------------------------------------------------------------- k-means++ on the device
@@ -506,22 +469,18 @@ def test_cuda_graph_replay_of_the_assignment_pass(ours, monkeypatch):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("n", [75776 + 2 * 128 + 17, 75776 + 4 * 128])   # 595 tiles (odd: phantom tile in the last pair) and 596
-def test_cta_pair_pass_equals_single_cta_pass_and_reference(ours, ref, monkeypatch, n):
+@pytest.mark.parametrize("n", cases.CTA_PAIR_ROWS)
+def test_cta_pair_pass_equals_single_cta_pass_and_reference(ours, monkeypatch, n):
     """The Lloyd pass runs as clusters of two CTAs (tcgen05.mma.cta_group::2, M = 256) once there are enough sample
     tiles; an odd tile count leaves a phantom tile in the last pair.  Both launch modes must give the reference's
     assignments (reference src/kmeans.cu:293-364)."""
-    rng = np.random.default_rng(4242)
-    d, k = 256, 1000          # K % 128 != 0: padded table rows in the last n-tile of both CTAs' halves
-    X = rng.random((n, d), dtype=np.float32)
-    C = X[rng.choice(n, k, replace=False)].copy()
-    _, a_ref = c_kmeans(ref, X, C, 1.0, 0.0)
+    X, C = cases.uniform_rows(n, 256, 1000, 4242)   # K % 128 != 0: padded table rows in the last n-tile of both halves
     got = {}
     for mode in ("1", "0"):
         monkeypatch.setenv("KMCUDA_B200_PAIR", mode)
         _, a = c_kmeans(ours, X, C, 1.0, 0.0)
         got[mode] = a
-        assert np.array_equal(a, a_ref), "pair=%s: %d assignments differ from the reference" % (mode, int((a != a_ref).sum()))
+        assert cases.digest(a) == str(REF["cta_pair/%d" % n]), "pair=%s: the assignments differ from the reference" % mode
     assert np.array_equal(got["1"], got["0"])
 
 
