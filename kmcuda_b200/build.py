@@ -48,15 +48,7 @@ def _run(cmd):
     return r.stdout
 
 
-def build(force=False, verbose=False, variant=None, defines=()):
-    """variant: build an A/B copy into variants/<variant>/libKMCUDA.so with extra -D defines (kernel tuning
-    experiments; select it at run time with KMCUDA_B200_LIB=<path>).  The product library is the default build."""
-    global OBJ, LIB
-    if variant:
-        vdir = os.path.join(ROOT, "variants", variant)
-        OBJ, LIB = os.path.join(vdir, "build"), os.path.join(vdir, "libKMCUDA.so")
-    else:
-        OBJ, LIB = os.path.join(HERE, "build"), os.path.join(HERE, "libKMCUDA.so")
+def build(force=False, verbose=False):
     os.makedirs(OBJ, exist_ok=True)
     headers = _headers()
     jobs = []
@@ -66,7 +58,7 @@ def build(force=False, verbose=False, variant=None, defines=()):
         o = os.path.join(OBJ, src + ".o")
         objs.append(o)
         if force or _newer(o, [s] + headers):
-            jobs.append([NVCC] + NVCC_FLAGS + ["-D" + d for d in defines] + ["-c", s, "-o", o])
+            jobs.append([NVCC] + NVCC_FLAGS + ["-c", s, "-o", o])
     for src in CC_SOURCES:
         s = os.path.join(CSRC, src)
         if not os.path.exists(s):
@@ -92,7 +84,5 @@ if __name__ == "__main__":
     import argparse
     ap = argparse.ArgumentParser()
     ap.add_argument("--force", action="store_true")
-    ap.add_argument("--variant", default=None)
-    ap.add_argument("-D", dest="defines", action="append", default=[])
     a = ap.parse_args()
-    print(build(force=a.force, verbose=True, variant=a.variant, defines=a.defines))
+    print(build(force=a.force, verbose=True))

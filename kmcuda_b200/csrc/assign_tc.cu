@@ -66,16 +66,10 @@ constexpr int TN = 128;                 // centroids per n-tile (UMMA N)
 constexpr int KB = 64;                  // fp16 elements per K-block = one 128-byte swizzle row of B
 constexpr int MAX_NKB = 8;              // D <= 512: A needs 32 TMEM columns per K-block; double-buffered up to 4 K-blocks
 constexpr int X_STAGES = 4;             // fp32 sample stages: 32 features x 128 rows = 16 KiB
-#ifndef KMB_B_STAGES
-#define KMB_B_STAGES 5
-#endif
-constexpr int B_STAGES = KMB_B_STAGES;  // fp16 centroid stages of ONE K-block (64 features x 128 rows = 16 KiB): a stage is
+constexpr int B_STAGES = 5;             // fp16 centroid stages of ONE K-block (64 features x 128 rows = 16 KiB): a stage is
                                         // refilled as soon as its 4 MMAs retire; 4 stages x 256 MMA cycles in flight cover
                                         // the L2 round trip (round 1: 2 stages of 32 KiB left the MMA warp waiting)
-#ifndef KMB_B_STAGES_PAIR
-#define KMB_B_STAGES_PAIR 8
-#endif
-constexpr int B_STAGES_PAIR = KMB_B_STAGES_PAIR;        // CTA-pair mode (cta_group::2): every CTA stages HALF a centroid tile per K-block, 8 KiB
+constexpr int B_STAGES_PAIR = 8;        // CTA-pair mode (cta_group::2): every CTA stages HALF a centroid tile per K-block, 8 KiB
 constexpr int B_STAGES_MAX = B_STAGES > B_STAGES_PAIR ? B_STAGES : B_STAGES_PAIR;
 constexpr int X_STAGE_BYTES = TM * 128;
 constexpr int B_KB_BYTES = TN * 128;     // one K-block of the centroid tile: 16 KiB
@@ -86,36 +80,13 @@ constexpr int LIST_LEN = 5;             // entries per epilogue thread: one per 
 // Warp roles.  The SM's issue arbiter prefers the highest warp id of a scheduler (B300_MICROARCH.md), so the warp
 // whose stalls cost tensor-pipe time -- the MMA issuer -- gets the highest id and the warps with slack (emitters)
 // the lowest.  Converter / epilogue warps keep warp % 4 = TMEM lane quarter.
-#ifndef KMB_ROLE_ORDER
-#define KMB_ROLE_ORDER 1
-#endif
-// Knock-out builds (timing experiments only, results are garbage): 1 = epilogue does not read the accumulators,
-// 2 = no MMA is issued, 3 = converters do no work (no LDS / math / tcgen05.st), 5 = the B / bias copies are not issued,
-// 6 = the X copies are not issued, 7 = the epilogue loads the accumulators but skips the ALU work on them.  Which of them shortens the kernel says what bounds it.
-#ifndef KMB_KO
-#define KMB_KO 0
-#endif
-// MMA issuer warps: ONE.  (Round 2 measured a second issuer taking alternate n-tiles: it helped the whole-warp
-// elect-per-K-block issue loop, 5.05 -> 4.40 ms, and hurts the lean single-thread loop, 3.88 -> 4.29 ms: with two n-tiles
-// in flight the 5-stage B ring, 1.25 n-tiles deep, becomes the limit.)  KMB_MMA_WARPS=2 keeps the variant buildable.
-#ifndef KMB_PREP_FUSED
-#define KMB_PREP_FUSED 1   // 1: centroid preparation as one launch (tc_prep_fused_kernel), 0: the chain of small kernels
-#endif
-#ifndef KMB_MMA_WARPS
-#define KMB_MMA_WARPS 1
-#endif
-constexpr int N_MMA_WARPS = KMB_MMA_WARPS;
-#if KMB_ROLE_ORDER == 1
+// There is ONE MMA issuer: round 2 measured a second one taking alternate n-tiles, and with the lean single-thread issue
+// loop it was slower (3.88 -> 4.29 ms), because with two n-tiles in flight the 5-stage B ring, 1.25 n-tiles deep,
+// becomes the limit.
 constexpr int FIRST_EMIT_WARP = 0;      // 4 emitter warps (merge + global emission)
 constexpr int FIRST_CONV_WARP = 4;      // 4 converter warps, warp % 4 = TMEM lane quarter
 constexpr int FIRST_EPI_WARP = 8;       // 8 epilogue warps
-constexpr int WARP_B_PRODUCER = 16, WARP_X_PRODUCER = 17, WARP_MMA = 19, WARP_MMA2 = 18;
-#else
-constexpr int WARP_B_PRODUCER = 0, WARP_MMA = 1, WARP_X_PRODUCER = 2, WARP_MMA2 = 3;
-constexpr int FIRST_CONV_WARP = 4;
-constexpr int FIRST_EPI_WARP = 8;
-constexpr int FIRST_EMIT_WARP = 16;
-#endif
+constexpr int WARP_B_PRODUCER = 16, WARP_X_PRODUCER = 17, WARP_MMA = 19;
 constexpr int N_CONV_WARPS = 4;
 constexpr int N_EPI_WARPS = 8;
 constexpr int N_EMIT_WARPS = 4;
@@ -255,7 +226,6 @@ struct Params {
   float* knn_dub;                // [stride] upper bound of the exact distance to the kk-th nearest candidate seen so far
   uint4* knn_entries;            // [stride][KNN_CAP]: (group max bits (g-space), mask, chunk id, margin bits)
   uint32_t knn_part, knn_nparts; // query-tile shard of this device (0, 1 = everything)
-  float* dbg_scores;         // optional [ntiles*128][nt*128] dump of the approximate scores
 };
 
 // ---------------------------------------------------------------------------------------------------
@@ -272,81 +242,7 @@ __global__ void tc_prep_stats_kernel(const float* __restrict__ csq, uint32_t K, 
   if ((threadIdx.x & 31) == 0) atomicMax(&st->csq_max_bits, best);
 }
 
-// cosine: upper bound of ||c||^2 per centroid (one warp per row)
-// (k-NN: the "centroids" are the samples in cluster-sorted order, row r = C[gather[r]], and the value feeds the bias
-// term, so no safety factor is applied)
-__global__ void tc_prep_norms_kernel(const float* __restrict__ C, uint32_t K, int D, float* __restrict__ out,
-                                     const uint32_t* __restrict__ gather, float factor) {
-  const uint32_t row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  if (row >= K) return;
-  const float* src = C + static_cast<size_t>(gather ? gather[row] : row) * D;
-  float a = 0.f;
-  for (int f = lane; f < D; f += 32) {
-    float v = src[f];
-    a = fmaf(v, v, a);
-  }
-  for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
-  if (lane == 0) out[row] = a * factor;
-}
-
-// centring vector of the L2 filter: column sums of the valid centroids (rows whose ||c||^2 is finite).  ANY vector
-// is a correct choice of mu (scores shift by a per-row constant); the mean minimises the operand norms.
-__global__ void tc_prep_mean_kernel(const float* __restrict__ C, const float* __restrict__ csq, uint32_t K, int D,
-                                    double* __restrict__ musum, uint32_t* __restrict__ nvalid) {
-  const int f = blockIdx.x * blockDim.x + threadIdx.x;
-  const uint32_t r0 = blockIdx.y * 64u, r1 = min(K, r0 + 64u);
-  double a = 0.0;
-  uint32_t nv = 0;
-  // 8 rows per step, loads first: the 64 rows of a CTA were one chain of dependent global loads before (36 us per pass)
-  for (uint32_t rb = r0; rb < r1; rb += 8) {
-    float v[8], q[8];
-#pragma unroll
-    for (int j = 0; j < 8; j++) {
-      const uint32_t r = min(rb + j, r1 - 1);
-      q[j] = csq[r];
-      v[j] = f < D ? C[static_cast<size_t>(r) * D + f] : 0.f;
-    }
-#pragma unroll
-    for (int j = 0; j < 8; j++) {
-      if (rb + j >= r1 || !(q[j] == q[j] && q[j] < 3.0e38f)) continue;
-      nv++;
-      a += static_cast<double>(v[j]);
-    }
-  }
-  if (f < D && nv) atomicAdd(&musum[f], a);
-  if (blockIdx.x == 0 && threadIdx.x == 0 && nv) atomicAdd(nvalid, nv);
-}
-__global__ void tc_prep_mu_kernel(const double* __restrict__ musum, const uint32_t* __restrict__ nvalid, int D,
-                                  float* __restrict__ mu) {
-  const int f = blockIdx.x * blockDim.x + threadIdx.x;
-  if (f >= D) return;
-  const uint32_t nv = *nvalid;
-  const float m = nv ? static_cast<float>(musum[f] / nv) : 0.f;
-  mu[f] = (fabsf(m) < 3.0e38f) ? m : 0.f;
-}
-// ||c - mu||^2 per centroid (one warp per row, double accumulation: the value becomes the bias term)
-__global__ void tc_prep_cnorm_kernel(const float* __restrict__ C, const float* __restrict__ csq,
-                                     const float* __restrict__ mu, uint32_t K, int D, float* __restrict__ out) {
-  const uint32_t row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  if (row >= K) return;
-  const float* src = C + static_cast<size_t>(row) * D;
-  double a = 0.0;
-  for (int f = lane; f < D; f += 32) {
-    const float v = src[f] - mu[f];      // the fp32 difference IS the table operand (before scaling)
-    a += static_cast<double>(v) * v;
-  }
-  for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
-  if (lane == 0) {
-    const float q = csq[row];
-    out[row] = (q == q && q < 3.0e38f) ? static_cast<float>(a) : q;   // dead centroids stay dead
-  }
-}
-
-__global__ void tc_prep_scale_kernel(Stats* __restrict__ st, const float* __restrict__ mu, int D, int Dp,
-                                     float* __restrict__ neg_mu_s) {   // one warp
-  const int lane = threadIdx.x;
+__global__ void tc_prep_scale_kernel(Stats* __restrict__ st) {   // one thread
   float cmax = __fsqrt_ru(__uint_as_float(st->csq_max_bits));
   float s = 1.f;
   if (cmax > 0.f && cmax < 3.0e38f) {
@@ -354,20 +250,9 @@ __global__ void tc_prep_scale_kernel(Stats* __restrict__ st, const float* __rest
     frexpf(cmax, &e);          // cmax = m * 2^e, m in [0.5, 1)
     s = ldexpf(1.f, 6 - e);    // s*cmax in [32, 64)
   }
-  float m2 = 0.f;
-  if (neg_mu_s)
-    for (int f = lane; f < Dp; f += 32) {
-      const float m = (mu && f < D) ? mu[f] : 0.f;
-      neg_mu_s[f] = -m * s;      // exact (power of two) unless it overflows, which the norm below reports
-      m2 = fmaf(m * s, m * s, m2);
-    }
-  for (int o = 16; o > 0; o >>= 1) m2 += __shfl_xor_sync(0xffffffffu, m2, o);
-  if (lane == 0) {
-    st->scale = s;
-    st->cmax = cmax * s * 1.001f;
-    st->dcmax = 0.f;
-    st->mun = __fsqrt_ru(m2) * 1.002f;   // (1.002: the lane-partial sums are added in a different order than a serial loop)
-  }
+  st->scale = s;
+  st->cmax = cmax * s * 1.001f;
+  st->dcmax = 0.f;
 }
 
 // one table row (a centroid, or a zero padding row up to nt*TN) by one warp; s = Stats::scale; csq / mu may have been
@@ -450,36 +335,23 @@ __device__ __forceinline__ void prep_table_row(uint32_t row, int lane, float s, 
   }
 }
 
-// one warp per centroid row (including the zero padding rows up to nt*256)
-__global__ void tc_prep_table_kernel(int metric, const float* __restrict__ C, const float* __restrict__ csq,
-                                     uint32_t K, int D, int nkb, int nt, __half* __restrict__ table,
-                                     __half* __restrict__ aug_blob, Stats* __restrict__ st,
-                                     const uint32_t* __restrict__ gather, const float* __restrict__ mu,
-                                     int by_source, int pair_blob = 0) {
-  const uint32_t row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  if (row >= static_cast<uint32_t>(nt) * TN) return;
-  prep_table_row(row, lane, st->scale, metric, C, csq, K, D, nkb, table, aug_blob, st, gather, mu, by_source, pair_blob);
-}
-
 // ---------------------------------------------------------------------------------------------------
 // The whole centroid preparation of one pass as ONE launch (Lloyd / Yinyang tables; the k-NN tables have their own
-// chain).  The chain above is ten stream operations (three memsets, ||c||^2, mean, mu, centred norms, maximum, scale,
-// table) of 3-12 us each on a 1 MB centroid matrix: ~0.05 ms of dependent launches per pass, 1 % of the step of an
-// 8M-row shard and 8 % of the step of a 1M-row shard (8 GPUs).  Here the same arithmetic (the device bodies are shared
-// with the chain, which stays as the KMB_PREP_FUSED=0 build) runs as four phases of one small grid separated by a
-// sense-reversing grid barrier; every CTA is resident (grid <= number of SMs, 256 threads, 34 KB static shared memory),
+// kernels).  As a chain of small kernels it was ten stream operations (three memsets, ||c||^2, mean, mu, centred norms,
+// maximum, scale, table) of 3-12 us each on a 1 MB centroid matrix: ~0.05 ms of dependent launches per pass, 1 % of the
+// step of an 8M-row shard and 8 % of the step of a 1M-row shard (8 GPUs), as measured in round 2; that chain has since
+// been removed.  Here the same arithmetic runs as four phases of one small grid separated by a sense-reversing grid
+// barrier; every CTA is resident (grid <= number of SMs, 256 threads, 34 KB static shared memory),
 // so the barrier cannot deadlock.  Values produced by other CTAs in an earlier phase are read with ld.global.cg.
 // ---------------------------------------------------------------------------------------------------
 struct PrepArgs {
-  int metric, centred, D, nkb, by_source, pair_blob;
+  int metric, D, nkb, by_source, pair_blob;
   uint32_t K, rows_pad;
   const float* C;
   float* csq;            // reference-order ||c||^2 (L2) / 1 (cosine); written here when compute_csq
   int compute_csq;
-  float* cnorm2;         // L2 centred: ||c - mu||^2; cosine: upper bound of ||c||^2
+  float* cnorm2;         // L2: ||c - mu||^2; cosine: upper bound of ||c||^2
   double* musum;         // [D] + valid-row count
-  float* mu;             // [D]
   float* neg_mu_s;       // [nkb * KB]
   Stats* stats;
   uint32_t* counters;    // CNT_N words, zeroed here
@@ -521,7 +393,7 @@ tc_prep_fused_kernel(const PrepArgs a) {
   // ---- phase 0: zero the pass counters / statistics / column sums; ||c||^2 in the reference's order
   if (gt < CNT_N) a.counters[gt] = 0u;
   if (gt < sizeof(Stats) / 4) reinterpret_cast<uint32_t*>(a.stats)[gt] = 0u;
-  if (a.centred)
+  if (a.metric == 0)
     for (uint32_t i = gt; i < static_cast<uint32_t>(D) + 1u; i += nthr) a.musum[i] = 0.0;
   if (a.compute_csq) {
     float* tile = s_tile[warp];
@@ -563,7 +435,7 @@ tc_prep_fused_kernel(const PrepArgs a) {
 
   const float* nsq = a.csq;
   if (a.metric == 1) {
-    // ---- cosine: upper bound of ||c||^2 per centroid + its maximum (tc_prep_norms_kernel, tc_prep_stats_kernel)
+    // ---- cosine: upper bound of ||c||^2 per centroid (one warp per row) + its maximum
     uint32_t best = 0;
     for (uint32_t row = gw; row < K; row += nw) {
       const float* src = a.C + static_cast<size_t>(row) * D;
@@ -580,8 +452,9 @@ tc_prep_fused_kernel(const PrepArgs a) {
     if (lane == 0 && best) atomicMax(&a.stats->csq_max_bits, best);
     nsq = a.cnorm2;
     prep_grid_barrier(a.barrier, gridDim.x);
-  } else if (a.centred) {
-    // ---- phase 1: column sums of the valid centroids (as tc_prep_mean_kernel: 128 features per half CTA)
+  } else {
+    // ---- phase 1: column sums of the valid centroids (rows whose ||c||^2 is finite), 128 features per half CTA.  ANY
+    // vector is a correct choice of mu (scores shift by a per-row constant); the mean minimises the operand norms.
     {
       const int fb = (D + 127) / 128;
       const uint32_t nvb = static_cast<uint32_t>(fb) * ((K + 15u) / 16u);   // 16 rows per half CTA: two load groups deep
@@ -616,9 +489,7 @@ tc_prep_fused_kernel(const PrepArgs a) {
       const uint32_t nv = __ldcg(reinterpret_cast<const uint32_t*>(a.musum + D));
       for (int f = tid; f < D; f += 256) {
         const float m = nv ? static_cast<float>(__ldcg(a.musum + f) / nv) : 0.f;
-        const float mm = (fabsf(m) < 3.0e38f) ? m : 0.f;
-        s_mu[f] = mm;
-        if (blockIdx.x == 0) a.mu[f] = mm;
+        s_mu[f] = (fabsf(m) < 3.0e38f) ? m : 0.f;
       }
       __syncthreads();
       uint32_t best = 0;
@@ -639,20 +510,10 @@ tc_prep_fused_kernel(const PrepArgs a) {
     }
     nsq = a.cnorm2;
     prep_grid_barrier(a.barrier, gridDim.x);
-  } else {
-    // ---- uncentred L2 (A/B switch): maximum of ||c||^2
-    uint32_t best = 0;
-    for (uint32_t c = gt; c < K; c += nthr) {
-      const float v = __ldcg(a.csq + c);
-      if (v == v && v < 3.0e38f) best = max(best, __float_as_uint(fmaxf(v, 0.f)));
-    }
-    for (int o = 16; o > 0; o >>= 1) best = max(best, __shfl_xor_sync(0xffffffffu, best, o));
-    if (lane == 0 && best) atomicMax(&a.stats->csq_max_bits, best);
-    prep_grid_barrier(a.barrier, gridDim.x);
   }
 
   // ---- phase 3: scale (every CTA derives it; CTA 0 publishes Stats and -mu*s), then the fp16 table + bias blocks
-  const bool have_mu = a.metric == 0 && a.centred;
+  const bool have_mu = a.metric == 0;
   if (warp == 0) {
     float cmax = __fsqrt_ru(__uint_as_float(__ldcg(&a.stats->csq_max_bits)));
     float s = 1.f;
@@ -691,15 +552,6 @@ tc_prep_fused_kernel(const PrepArgs a) {
 // bars_u32 = shared-space address of bars[0] (computed once per thread)
 #define TC_WAIT(bar, parity, site) \
   ptx::mbar_wait(bars_u32 + 8u * static_cast<uint32_t>(bar), (parity), p.counters + CNT_ERR, site, bars_u32 + 8u * 63u)
-#ifndef KMB_MMA_SPIN
-#define KMB_MMA_SPIN 0
-#endif
-#if KMB_MMA_SPIN
-#define TC_WAIT_MMA(bar, parity, site) \
-  ptx::mbar_wait_spin(bars_u32 + 8u * static_cast<uint32_t>(bar), (parity), p.counters + CNT_ERR, site, bars_u32 + 8u * 63u)
-#else
-#define TC_WAIT_MMA TC_WAIT
-#endif
 
 // the reference's bookkeeping for one decided row (kmeans.cu:356-363); returns 1 if the assignment changed
 __device__ __forceinline__ uint32_t commit_assignment(uint32_t* __restrict__ assign, uint32_t* __restrict__ prev,
@@ -836,17 +688,9 @@ tc_assign_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_consta
   constexpr int nkb = NKB;
   constexpr int NBUF = NKB <= 4 ? 2 : 1;   // A operand buffers in TMEM (256 columns are available for A)
   // The error bound needs |x~| (the fp16-rounded operand row) and the rounding residual |a - x~|; the converters MEASURE
-  // both.  KMB_ANALYTIC_RESIDUAL=1 (A/B build) bounds them from |a|^2 alone in the streaming modes 0 and 3 -- round-to-
-  // nearest into fp16 moves a normal value by at most 2^-11 |a_i|, a subnormal one by at most 2^-25 -- which takes the
-  // back-conversion and the residual sums out of the converter's inner loop (17 -> 9 instructions per 4 elements).
-  // Measured at 8M x 256 @ 1024: the kernel time does not change (the converters are not on the critical path) while the
-  // margin widens and 8.1 % instead of 5.0 % of the rows need the exact re-check, so it is off.
-#if defined(KMB_ANALYTIC_RESIDUAL) && KMB_ANALYTIC_RESIDUAL
-  constexpr bool MEASURED_RESIDUAL = (MODE == 1 || MODE == 2);
-#else
-  constexpr bool MEASURED_RESIDUAL = true;
-#endif
-  [[maybe_unused]] const int nt = p.nt;
+  // both.  Round 2 measured bounding them analytically from |a|^2 instead, at 8M x 256 @ 1024: the kernel time did not
+  // change (the converters are not on the critical path) while the margin widened and 8.1 % instead of 5.0 % of the
+  // rows needed the exact re-check.
   const uint32_t n_eff = MODE == 1 ? min(*p.d_nrows, p.n) : p.n;
   const uint32_t ntiles = MODE == 1 ? (n_eff + TM - 1) / TM : (MODE == 2 ? *p.d_ntiles : p.ntiles);
   // MODE 2 on several GPUs: this device serves the query tiles of part knn_part of knn_nparts (every GPU holds the
@@ -879,7 +723,7 @@ tc_assign_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_consta
       ptx::mbar_init(&bars[BAR_AUG_EMPTY + s], 1);
       ptx::mbar_init(&bars[BAR_ACC_FULL + s], 1);
       ptx::mbar_init(&bars[BAR_ACC_EMPTY + s], N_EPI_WARPS * CG);   // pair: the leader's barrier counts both CTAs' warps
-      ptx::mbar_init(&bars[BAR_A_FREE + s], N_MMA_WARPS);
+      ptx::mbar_init(&bars[BAR_A_FREE + s], 1);
       ptx::mbar_init(&bars[BAR_EMIT_FULL + s], N_EPI_WARPS);
       ptx::mbar_init(&bars[BAR_EMIT_EMPTY + s], N_EMIT_WARPS);
       for (int kb = 0; kb < MAX_NKB; kb++) ptx::mbar_init(&bars[BAR_A_FULL + s * MAX_NKB + kb], N_CONV_WARPS * CG);
@@ -927,14 +771,10 @@ tc_assign_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_consta
             ptx::tma_load_2d_pair(ptx::smem_u32(smem + L.aug_b + as * AUG_B_BYTES), &tmap_aug, 0,
                                   (n * 2 + static_cast<int>(cta_rank)) * 2, leader_bar(BAR_AUG_FULL + as));
           } else {
-#if KMB_KO == 5
-          ptx::mbar_arrive(&bars[BAR_AUG_FULL + as]);
-#else
-          ptx::mbar_arrive_expect_tx(&bars[BAR_AUG_FULL + as], AUG_B_BYTES);
-          ptx::bulk_load(smem + L.aug_b + as * AUG_B_BYTES,
-                         reinterpret_cast<const uint8_t*>(p.aug_blob) + static_cast<size_t>(n) * AUG_B_BYTES,
-                         AUG_B_BYTES, &bars[BAR_AUG_FULL + as]);
-#endif
+            ptx::mbar_arrive_expect_tx(&bars[BAR_AUG_FULL + as], AUG_B_BYTES);
+            ptx::bulk_load(smem + L.aug_b + as * AUG_B_BYTES,
+                           reinterpret_cast<const uint8_t*>(p.aug_blob) + static_cast<size_t>(n) * AUG_B_BYTES,
+                           AUG_B_BYTES, &bars[BAR_AUG_FULL + as]);
           }
           ac++;
 #pragma unroll
@@ -945,12 +785,8 @@ tc_assign_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_consta
               ptx::tma_load_2d_pair(ptx::smem_u32(smem + L.b + bs * BSTAGE), &tmap_b, kb * KB,
                                     n * TN + static_cast<int>(cta_rank) * (TN / 2), leader_bar(BAR_B_FULL + bs));
             } else {
-#if KMB_KO == 5
-            ptx::mbar_arrive(&bars[BAR_B_FULL + bs]);
-#else
-            ptx::mbar_arrive_expect_tx(&bars[BAR_B_FULL + bs], B_KB_BYTES);
-            ptx::tma_load_2d(smem + L.b + bs * B_STAGE_BYTES, &tmap_b, kb * KB, n * TN, &bars[BAR_B_FULL + bs]);
-#endif
+              ptx::mbar_arrive_expect_tx(&bars[BAR_B_FULL + bs], B_KB_BYTES);
+              ptx::tma_load_2d(smem + L.b + bs * B_STAGE_BYTES, &tmap_b, kb * KB, n * TN, &bars[BAR_B_FULL + bs]);
             }
             if (++bs == BST) { bs = 0; bph ^= 1; }
           }
@@ -966,29 +802,22 @@ tc_assign_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_consta
           const int s = xc % X_STAGES;
           const uint32_t ph = (xc / X_STAGES) & 1;
           TC_WAIT(BAR_X_EMPTY + s, ph ^ 1, 9);
-#if KMB_KO == 6
-          ptx::mbar_arrive(&bars[BAR_X_FULL + s]);
-#else
           ptx::mbar_arrive_expect_tx(&bars[BAR_X_FULL + s], X_STAGE_BYTES);
           ptx::tma_load_2d(smem + L.x + s * X_STAGE_BYTES, &tmap_x, hs * 32, static_cast<int>(tile * TM),
                            &bars[BAR_X_FULL + s]);
-#endif
         }
       }
     }
-  } else if (warp == WARP_MMA || (N_MMA_WARPS == 2 && warp == WARP_MMA2)) {
-    // ================================ MMA issuer(s) ================================
-    // ONE thread per issuer warp runs the whole role (tcgen05.mma / commit are single-thread instructions): no
-    // election, no reconvergence points, no warp-wide barrier probes.  ncu of the previous version (whole warp +
-    // elect per K-block, profiles/r02_tc_assign_v6_*): ~330 SASS instructions per n-tile at ~6 cycles each = ~2000
-    // cycles to issue 1088 cycles of tensor work -- the issuer, not the tensor pipe, paced the kernel.  Descriptors are
-    // built once; a K-block is one asm statement (4 MMAs + commit).
-    // With two issuers every issuer walks all n-tiles (so the ring / buffer counters stay in step) but issues only
-    // the n-tiles whose accumulator buffer it owns (n-tile counter & 1 == me).
+  } else if (warp == WARP_MMA) {
+    // ================================ MMA issuer ================================
+    // ONE thread runs the whole role (tcgen05.mma / commit are single-thread instructions): no election, no
+    // reconvergence points, no warp-wide barrier probes.  ncu of the previous version (whole warp + elect per K-block,
+    // profiles/r02_tc_assign_v6_*): ~330 SASS instructions per n-tile at ~6 cycles each = ~2000 cycles to issue 1088
+    // cycles of tensor work -- the issuer, not the tensor pipe, paced the kernel.  Descriptors are built once; a K-block
+    // is one asm statement (4 MMAs + commit).
     // CTA pairs: only the leader issues (M = 256 covers both CTAs' rows); its commits are multicast to both CTAs.
     if ((!PAIR || cta_rank == 0) && ptx::elect_one()) {   // (elect.sync, not `lane == 0`: ptxas then keeps the operands in
                               // uniform registers instead of wrapping every tcgen05 instruction in a per-lane R2UR.BROADCAST loop)
-      const uint32_t me = (warp == WARP_MMA) ? 0u : 1u;
       const uint32_t idesc = ptx::make_idesc_f16(TM * CG, TN);
       const uint64_t bdesc0 = ptx::make_smem_desc(ptx::smem_u32(smem + L.b), 16, 1024, 2);
       const uint64_t aug_ad = ptx::make_smem_desc(ptx::smem_u32(smem + L.aug_a), TM * 16, 128, 0);
@@ -999,60 +828,44 @@ tc_assign_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_consta
         else ptx::umma_commit_u32(bars_u32 + 8u * static_cast<uint32_t>(bar));
       };
       uint32_t bs = 0, bph = 0, ac = 0, si = 0;             // B ring stage / phase; n-tiles; segments (= A conversions) so far
-      uint32_t a_ready_si = 0xFFFFFFFFu;                    // segment whose A operand this issuer has already waited for
-      bool issued = false;                                  // this issuer has MMAs in flight that read the current A buffer
+      uint32_t a_ready_si = 0xFFFFFFFFu;                    // segment whose A operand has already been waited for
       for (uint32_t tile = tile_begin; tile < tile_end; tile += gridDim.x) {
         if (MODE == 2 && p.knn_nblk[tile] == 0) continue;   // nothing to visit: every role skips the tile
         for (BlockIter<MODE> it(p, tile); it.valid(); it.next(), ac++) {
-          const bool mine = N_MMA_WARPS == 1 || (ac & 1u) == me;
           const uint32_t abuf = si % NBUF;
           const uint32_t a_par = (si / NBUF) & 1;
           const uint32_t buf = ac & 1;
           const uint32_t aph = (ac >> 1) & 1;
-          if (mine) {
-            const bool need_a = a_ready_si != si;           // first n-tile of this segment that THIS issuer multiplies
-            a_ready_si = si;
-            const uint32_t a_tmem = tmem_base + TMEM_A0 + abuf * 128;
-            const uint32_t d_tmem = tmem_base + TMEM_ACC0 + buf * TN;
-            TC_WAIT_MMA(BAR_ACC_EMPTY + buf, aph ^ 1, 3);
-            uint32_t s_ = bs, ph_ = bph;
+          const bool need_a = a_ready_si != si;             // first n-tile of this segment
+          a_ready_si = si;
+          const uint32_t a_tmem = tmem_base + TMEM_A0 + abuf * 128;
+          const uint32_t d_tmem = tmem_base + TMEM_ACC0 + buf * TN;
+          TC_WAIT(BAR_ACC_EMPTY + buf, aph ^ 1, 3);
+          uint32_t s_ = bs, ph_ = bph;
 #pragma unroll
-            for (int kb = 0; kb < NKB; kb++) {
-              if (need_a) TC_WAIT_MMA(BAR_A_FULL + abuf * MAX_NKB + kb, a_par, 4);
-              TC_WAIT_MMA(BAR_B_FULL + s_, ph_, 5);
-              ptx::tc_fence_after();
-#if KMB_KO != 2
-              if (PAIR)
-                ptx::umma_f16_ts_kblock_pair(d_tmem, a_tmem + kb * 32, bdesc0 + s_ * (BSTAGE >> 4), idesc, kb ? 1u : 0u,
-                                             bars_u32 + 8u * (BAR_B_EMPTY + s_));
-              else
-                ptx::umma_f16_ts_kblock(d_tmem, a_tmem + kb * 32, bdesc0 + s_ * (BSTAGE >> 4), idesc, kb ? 1u : 0u,
-                                        bars_u32 + 8u * (BAR_B_EMPTY + s_));
-#else
-              commit(BAR_B_EMPTY + s_);
-#endif
-              if (++s_ == BST) { s_ = 0; ph_ ^= 1; }
-            }
-            // bias step: acc += ones(128x16) * bias(128x16)^T  (both operands no-swizzle K-major smem blocks)
-            TC_WAIT_MMA(BAR_AUG_FULL + buf, aph, 6);
+          for (int kb = 0; kb < NKB; kb++) {
+            if (need_a) TC_WAIT(BAR_A_FULL + abuf * MAX_NKB + kb, a_par, 4);
+            TC_WAIT(BAR_B_FULL + s_, ph_, 5);
             ptx::tc_fence_after();
-#if KMB_KO != 2
-            if (PAIR) ptx::umma_f16_pair(d_tmem, aug_ad, aug_bd0 + buf * (AUG_B_BYTES >> 4), idesc, 1u);
-            else ptx::umma_f16(d_tmem, aug_ad, aug_bd0 + buf * (AUG_B_BYTES >> 4), idesc, 1u);
-#endif
-            commit(BAR_AUG_EMPTY + buf);
-            commit(BAR_ACC_FULL + buf);
-            issued = true;
+            if (PAIR)
+              ptx::umma_f16_ts_kblock_pair(d_tmem, a_tmem + kb * 32, bdesc0 + s_ * (BSTAGE >> 4), idesc, kb ? 1u : 0u,
+                                           bars_u32 + 8u * (BAR_B_EMPTY + s_));
+            else
+              ptx::umma_f16_ts_kblock(d_tmem, a_tmem + kb * 32, bdesc0 + s_ * (BSTAGE >> 4), idesc, kb ? 1u : 0u,
+                                      bars_u32 + 8u * (BAR_B_EMPTY + s_));
+            if (++s_ == BST) { s_ = 0; ph_ ^= 1; }
           }
-          // the B ring advances by one n-tile for every issuer
+          // bias step: acc += ones(128x16) * bias(128x16)^T  (both operands no-swizzle K-major smem blocks)
+          TC_WAIT(BAR_AUG_FULL + buf, aph, 6);
+          ptx::tc_fence_after();
+          if (PAIR) ptx::umma_f16_pair(d_tmem, aug_ad, aug_bd0 + buf * (AUG_B_BYTES >> 4), idesc, 1u);
+          else ptx::umma_f16(d_tmem, aug_ad, aug_bd0 + buf * (AUG_B_BYTES >> 4), idesc, 1u);
+          commit(BAR_AUG_EMPTY + buf);
+          commit(BAR_ACC_FULL + buf);
           bs += NKB;
           while (bs >= static_cast<uint32_t>(BST)) { bs -= BST; bph ^= 1; }
           if (it.seg_last()) {
-            // the A buffer of this segment is free once BOTH issuers' MMAs on it have retired: a commit tracks only the
-            // issuing thread's own MMAs, so every issuer arrives (a plain arrive if it multiplied nothing here)
-            if (issued) commit(BAR_A_FREE + abuf);
-            else ptx::mbar_arrive_u32(bars_u32 + 8u * (BAR_A_FREE + abuf));
-            issued = false;
+            commit(BAR_A_FREE + abuf);   // the A buffer of this segment is free once its MMAs have retired
             si++;
           }
         }
@@ -1102,7 +915,7 @@ tc_assign_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_consta
             }
             const uint8_t* xs = smem + L.x + st * X_STAGE_BYTES + row * 128;
 #pragma unroll
-            for (int c = 0; c < (KMB_KO == 3 ? 0 : 8); c++) {
+            for (int c = 0; c < 8; c++) {
               float4 v = (MODE == 0 || MODE == 3) ? *reinterpret_cast<const float4*>(xs + ((c ^ (row & 7)) << 4)) : gv[c];
               float4 m4 = make_float4(0.f, 0.f, 0.f, 0.f);
               if (MODE == 2) {
@@ -1121,19 +934,13 @@ tc_assign_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_consta
               ptx::unpack2(a01, a0, a1);
               ptx::unpack2(a23, a2_, a3);
               __half2 h0 = __floats2half2_rn(a0, a1), h1 = __floats2half2_rn(a2_, a3);
-              if (MEASURED_RESIDUAL) {
-                const float2 b0 = __half22float2(h0), b1 = __half22float2(h1);
-                const uint64_t b01 = ptx::pack2(b0.x, b0.y), b23 = ptx::pack2(b1.x, b1.y);
-                nx2 = ptx::ffma2(b01, b01, nx2);
-                nx2 = ptx::ffma2(b23, b23, nx2);
-                const uint64_t d01 = ptx::fsub2(a01, b01), d23 = ptx::fsub2(a23, b23);
-                nd2 = ptx::ffma2(d01, d01, nd2);
-                nd2 = ptx::ffma2(d23, d23, nd2);
-              } else {
-                // |a|^2 before the rounding: the epilogue bounds the rounded norm and the residual from it
-                nx2 = ptx::ffma2(a01, a01, nx2);
-                nx2 = ptx::ffma2(a23, a23, nx2);
-              }
+              const float2 b0 = __half22float2(h0), b1 = __half22float2(h1);
+              const uint64_t b01 = ptx::pack2(b0.x, b0.y), b23 = ptx::pack2(b1.x, b1.y);
+              nx2 = ptx::ffma2(b01, b01, nx2);
+              nx2 = ptx::ffma2(b23, b23, nx2);
+              const uint64_t d01 = ptx::fsub2(a01, b01), d23 = ptx::fsub2(a23, b23);
+              nd2 = ptx::ffma2(d01, d01, nd2);
+              nd2 = ptx::ffma2(d23, d23, nd2);
               if (MODE == 2) {   // compensated: this sum is subtracted from scores of the same magnitude
                 const float q4 = fmaf(a0, a0, fmaf(a1, a1, fmaf(a2_, a2_, a3 * a3)));
                 const float y = q4 - a2c, t = a2 + y;
@@ -1148,19 +955,15 @@ tc_assign_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_consta
               if (lane == 0) ptx::mbar_arrive(&bars[BAR_X_EMPTY + st]);
             }
           }
-#if KMB_KO != 3
           ptx::tmem_st_32x32(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + TMEM_A0 + abuf * 128 + kb * 32, pk);
           ptx::tmem_st_wait();
-#else
-          (void)pk;
-#endif
           if (kb == nkb - 1) {
             float* norms = reinterpret_cast<float*>(smem + L.norms) + (si & 3) * 4 * TM;
             float nxl, nxh, ndl, ndh;
             ptx::unpack2(nx2, nxl, nxh);
             ptx::unpack2(nd2, ndl, ndh);
             norms[row] = nxl + nxh;
-            if (MEASURED_RESIDUAL) norms[TM + row] = ndl + ndh;
+            norms[TM + row] = ndl + ndh;
             if (MODE == 2) {
               norms[2 * TM + row] = a2;
               norms[3 * TM + row] = nraw * s * s;
@@ -1245,31 +1048,14 @@ tc_assign_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_consta
         // both 32-column chunks of this warp are fetched up front so that their dependency chains interleave
         uint32_t r0[32], r1[32];
         const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + TMEM_ACC0 + buf * TN + h * 64;
-#if KMB_KO != 1
         ptx::tmem_ld_32x32(taddr, r0);
         ptx::tmem_ld_32x32(taddr + 32, r1);
-#else
-        for (int jj = 0; jj < 32; jj++) {   // stand-in values: strictly decreasing, 64 apart -> one candidate per row
-          r0[jj] = __float_as_uint(-64.f * static_cast<float>(n * 128 + h * 64 + jj + 1));
-          r1[jj] = __float_as_uint(-64.f * static_cast<float>(n * 128 + h * 64 + 32 + jj + 1));
-        }
-#endif
         if (it.seg_first()) {
           const float* norms = reinterpret_cast<const float*>(smem + L.norms) + (si & 3) * 4 * TM;
           // rigorous bound on |acc - (s^2 x.c - s^2||c||^2/2)| (see header): Cauchy-Schwarz on the
           // actual rounding residuals + accumulation + the reference's own rounding slack
-          float nx, nd;
-          if (MEASURED_RESIDUAL) {
-            nx = __fsqrt_ru(norms[row]) * 1.0001f;
-            nd = __fsqrt_ru(norms[TM + row]) * 1.0001f;
-          } else {
-            // norms[row] = |a|^2 (fp32 sum, relative error < 1e-4): |a - x~| <= 2^-11 |a| + sqrt(Dp) 2^-25, |x~| <= |a| + |a - x~|
-            const float na = __fsqrt_ru(norms[row]) * 1.0001f;
-            nd = na * 4.8834e-4f + __fsqrt_ru(static_cast<float>(p.nkb * KB)) * 2.99e-8f;
-            nx = na + nd;
-            // an element beyond the fp16 range would have become Inf in the operand: such rows take the exact pass
-            if (!(na < 65000.f)) flags |= 1u;
-          }
+          const float nx = __fsqrt_ru(norms[row]) * 1.0001f;
+          const float nd = __fsqrt_ru(norms[TM + row]) * 1.0001f;
           const float xn = nx + nd;
           float E = nx * dcmax + nd * cmax + nd * dcmax;
           E += static_cast<float>(p.nkb * KB + 16) * 2.4e-7f * nx * cmax;   // fp32 accumulation in the tensor core
@@ -1324,14 +1110,6 @@ tc_assign_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_consta
           if (PAIR) ptx::mbar_arrive_cluster(leader_bar(BAR_ACC_EMPTY + buf));
           else ptx::mbar_arrive(&bars[BAR_ACC_EMPTY + buf]);
         }
-#ifdef KMB_DEBUG_SCORES   // bring-up builds only: 64 stores per n-tile bloat the hot loop's instruction footprint
-        if (MODE == 0 && p.dbg_scores) {
-          const uint64_t grow = static_cast<uint64_t>(tile) * TM + row;
-          float* dst = p.dbg_scores + grow * (static_cast<uint64_t>(nt) * TN) + n * TN + h * 64;
-          for (int jj = 0; jj < 32; jj++) dst[jj] = __uint_as_float(r0[jj]);
-          for (int jj = 0; jj < 32; jj++) dst[32 + jj] = __uint_as_float(r1[jj]);
-        }
-#endif
         if (MODE == 3) {
           // quad maxima (2 instructions per 4 columns), folded into per-group maxima along the (warp-uniform) group ids
           // of this 64-column half; every finished group turns into a lower bound of the distance
@@ -1385,16 +1163,6 @@ tc_assign_kernel(const __grid_constant__ CUtensorMap tmap_b, const __grid_consta
         // chunk maxima with three-input maxima (FMNMX3): 16 instructions per 32 columns
         float t0[8], t1[8];      // MODE 2 only: maxima of the 4-column groups
         float cm0, cm1;
-#if KMB_KO == 7
-        if (MODE == 0) {   // timing build: the accumulators are loaded, the ALU work on them is skipped
-          uint32_t x0 = 0, x1 = 0;
-#pragma unroll
-          for (int jj = 0; jj < 32; jj += 8) { x0 ^= r0[jj]; x1 ^= r1[jj]; }
-          M = fmaxf(M, __uint_as_float(x0 & x1 & 0x3fffffffu));
-          if (it.seg_last()) si++;
-          continue;
-        }
-#endif
         if (MODE == 2) {
 #pragma unroll
           for (int i = 0; i < 8; i++) {
@@ -1792,9 +1560,7 @@ struct TcPlan {
   tc::Stats* stats = nullptr;
   float* cnorm2 = nullptr;         // cosine: ||c||^2 (the reference's 'csqr' is the constant 1 there); L2: ||c - mu||^2
   double* musum = nullptr;         // [D] column sums of the valid centroids, followed by the valid-row count
-  float* mu = nullptr;             // [D] centring vector (L2), see Params::neg_mu_s
-  float* neg_mu_s = nullptr;       // [nkb*64]
-  bool centred = false;
+  float* neg_mu_s = nullptr;       // [nkb*64] L2: -mu*s with mu = mean of the valid centroids, see Params::neg_mu_s
   bool inject_error = false;       // test hook (KMCUDA_B200_INJECT_PIPELINE_ERROR=1): report a timed-out barrier
   // Yinyang bounds refresh (MODE 3): group-sorted table layout, built once per run by tc_yy_layout()
   int nt3 = 0;
@@ -1819,7 +1585,6 @@ struct TcPlan {
   CUtensorMap tmap_pair, tmap_aug;
   int num_sms = 148;
   size_t smem_bytes = 0;
-  float* dbg_scores = nullptr;
   // CUDA-event pairs around the main kernel of the most recent passes (bench.py roofline)
   static constexpr int kEvRing = 64;
   cudaEvent_t ev0[kEvRing] = {}, ev1[kEvRing] = {};
@@ -2011,7 +1776,6 @@ void tc_plan_destroy(TcPlan* p) {
   pool_free(p->stats);
   pool_free(p->cnorm2);
   pool_free(p->musum);
-  pool_free(p->mu);
   pool_free(p->neg_mu_s);
   pool_free(p->table3);
   pool_free(p->aug_blob3);
@@ -2026,7 +1790,6 @@ void tc_plan_destroy(TcPlan* p) {
   pool_free(p->ovf_rows);
   pool_free(p->counters);
   pool_free(p->prep_barrier);
-  pool_free(p->dbg_scores);
   pinned_counters_free(p->h_counters);
   for (int i = 0; i < TcPlan::kEvRing; i++) {
     if (p->ev0[i]) cudaEventDestroy(p->ev0[i]);
@@ -2055,11 +1818,8 @@ cudaError_t tc_plan_create(TcPlan** out, int metric, uint32_t max_n, int D, uint
   TC_TRY(pool_alloc(reinterpret_cast<void**>(&p->stats), sizeof(Stats)));
   TC_TRY(pool_alloc(reinterpret_cast<void**>(&p->cnorm2), sizeof(float) * K));
   TC_TRY(pool_alloc(reinterpret_cast<void**>(&p->musum), sizeof(double) * (D + 1)));
-  TC_TRY(pool_alloc(reinterpret_cast<void**>(&p->mu), sizeof(float) * D));
   TC_TRY(pool_alloc(reinterpret_cast<void**>(&p->neg_mu_s), sizeof(float) * MAX_NKB * KB));
   {
-    const char* nc = getenv("KMCUDA_B200_NO_CENTER");   // A/B switch: uncentred operands (the round-1 filter)
-    p->centred = metric == 0 && !(nc && nc[0] == '1');
     const char* ie = getenv("KMCUDA_B200_INJECT_PIPELINE_ERROR");
     p->inject_error = ie && ie[0] == '1';
   }
@@ -2075,11 +1835,6 @@ cudaError_t tc_plan_create(TcPlan** out, int metric, uint32_t max_n, int D, uint
   p->h_counters = pinned_counters_alloc();
   if (!p->h_counters) { tc_plan_destroy(p); return cudaErrorMemoryAllocation; }
   memset(p->h_counters, 0, sizeof(uint32_t) * CNT_N);
-  const char* dbg = getenv("KMCUDA_B200_DUMP_SCORES");
-  if (dbg && dbg[0] == '1') {
-    size_t tiles = (static_cast<size_t>(max_n) + TM - 1) / TM;
-    TC_TRY(pool_alloc(reinterpret_cast<void**>(&p->dbg_scores), tiles * TM * rows_pad * sizeof(float)));
-  }
   // tensor map over the fp16 centroid table [rows_pad][nkb*64], box 64 x 256, 128-byte swizzle
   EncodeTiledFn enc = get_encode_fn();
   if (!enc) { tc_plan_destroy(p); return cudaErrorNotSupported; }
@@ -2130,11 +1885,9 @@ static cudaError_t tc_prepare(TcPlan* p, const float* C, const float* csq, uint3
                               cudaStream_t st, bool yy_layout = false, bool pair_blob = false, bool compute_csq = false) {
   using namespace tc;
   cudaError_t e;
-#if KMB_PREP_FUSED
   {
     PrepArgs a;
     a.metric = p->metric;
-    a.centred = p->centred ? 1 : 0;
     a.D = p->D;
     a.nkb = p->nkb;
     a.by_source = yy_layout ? 1 : 0;
@@ -2146,7 +1899,6 @@ static cudaError_t tc_prepare(TcPlan* p, const float* C, const float* csq, uint3
     a.compute_csq = compute_csq ? 1 : 0;
     a.cnorm2 = p->cnorm2;
     a.musum = p->musum;
-    a.mu = p->mu;
     a.neg_mu_s = p->neg_mu_s;
     a.stats = p->stats;
     a.counters = p->counters;
@@ -2159,35 +1911,6 @@ static cudaError_t tc_prepare(TcPlan* p, const float* C, const float* csq, uint3
     tc_prep_fused_kernel<<<grid, 256, 0, st>>>(a);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
   }
-#else
-  if (compute_csq && (e = kmb::launch_csqr(p->metric, C, p->K, p->D, const_cast<float*>(csq), st)) != cudaSuccess) return e;
-  if ((e = cudaMemsetAsync(p->counters, 0, sizeof(uint32_t) * CNT_N, st)) != cudaSuccess) return e;
-  if ((e = cudaMemsetAsync(p->stats, 0, sizeof(Stats), st)) != cudaSuccess) return e;
-  const float* nsq = csq;
-  const float* mu = nullptr;
-  if (p->metric == 1) {
-    tc_prep_norms_kernel<<<(p->K * 32 + 255) / 256, 256, 0, st>>>(C, p->K, p->D, p->cnorm2, nullptr, 1.0001f);
-    nsq = p->cnorm2;
-  } else if (p->centred) {
-    // L2: both operands are centred on the mean of the valid centroids (see Params::neg_mu_s)
-    if ((e = cudaMemsetAsync(p->musum, 0, sizeof(double) * (p->D + 1), st)) != cudaSuccess) return e;
-    uint32_t* nvalid = reinterpret_cast<uint32_t*>(p->musum + p->D);
-    tc_prep_mean_kernel<<<dim3((p->D + 127) / 128, (p->K + 63) / 64), 128, 0, st>>>(C, csq, p->K, p->D, p->musum, nvalid);
-    tc_prep_mu_kernel<<<(p->D + 127) / 128, 128, 0, st>>>(p->musum, nvalid, p->D, p->mu);
-    tc_prep_cnorm_kernel<<<(p->K * 32 + 255) / 256, 256, 0, st>>>(C, csq, p->mu, p->K, p->D, p->cnorm2);
-    nsq = p->cnorm2;
-    mu = p->mu;
-  }
-  tc_prep_stats_kernel<<<8, 256, 0, st>>>(nsq, p->K, p->stats);
-  tc_prep_scale_kernel<<<1, 32, 0, st>>>(p->stats, mu, p->D, p->nkb * KB, p->neg_mu_s);
-  const uint32_t rows_pad = static_cast<uint32_t>(p->nt) * TN;
-  if (!yy_layout)
-    tc_prep_table_kernel<<<(rows_pad * 32 + 255) / 256, 256, 0, st>>>(p->metric, C, nsq, p->K, p->D, p->nkb, p->nt, p->table,
-                                                                      p->aug_blob, p->stats, nullptr, mu, 0, pair_blob ? 1 : 0);
-  else
-    tc_prep_table_kernel<<<(static_cast<uint32_t>(p->nt3) * TN * 32 + 255) / 256, 256, 0, st>>>(
-        p->metric, C, nsq, p->K, p->D, p->nkb, p->nt3, p->table3, p->aug_blob3, p->stats, p->yy_perm, mu, 1);
-#endif
   Params prm;
   prm.n = n;
   prm.D = p->D;
@@ -2229,7 +1952,6 @@ static cudaError_t tc_prepare(TcPlan* p, const float* C, const float* csq, uint3
   prm.knn_entries = nullptr;
   prm.knn_part = 0;
   prm.knn_nparts = 1;
-  prm.dbg_scores = p->dbg_scores;
   *out = prm;
   return cudaGetLastError();
 }
@@ -2579,10 +2301,6 @@ int tc_kernel_times(TcPlan* p, float* ms_out, int max_out) {
     ms_out[i] = ms;
   }
   return n;
-}
-const float* tc_debug_scores(TcPlan* p, size_t* row_stride) {
-  *row_stride = static_cast<size_t>(p->nt) * tc::TN;
-  return p->dbg_scores;
 }
 void tc_debug_stats(TcPlan* p, float* out4) {
   tc::Stats st;
@@ -3058,7 +2776,7 @@ cudaError_t tc_knn_search(int metric, int k, const float* X, const float* C, uin
   // fp16 table of the centred samples + bias blobs + statistics
   knn::prep_norms_kernel<<<(rows_max / 8) + 1, 256, 0, st>>>(X, C, D, tab2orig, blk_cluster, d_ntiles, ysq, yabs, metric);
   tc_prep_stats_kernel<<<8, 256, 0, st>>>(ysq, rows_max, stats);
-  tc_prep_scale_kernel<<<1, 32, 0, st>>>(stats, nullptr, 0, 0, nullptr);
+  tc_prep_scale_kernel<<<1, 1, 0, st>>>(stats);
   knn::prep_table_kernel<<<(rows_max / 8) + 1, 256, 0, st>>>(X, C, D, nkb, tab2orig, blk_cluster, d_ntiles, ysq, table,
                                                              blobs, stats, yabs, metric, d_err);
   KNN_TRY(cudaGetLastError());
@@ -3080,7 +2798,6 @@ cudaError_t tc_knn_search(int metric, int k, const float* X, const float* C, uin
   prm.knn_ranges = ranges1; prm.knn_roff = roff1; prm.knn_rcount = rcount1; prm.knn_nblk = nblk1;
   prm.kk = kk; prm.knn_first_pass = 1; prm.knn_stride = stride; prm.knn_topk = topk;
   prm.knn_cnt = kcnt; prm.knn_flags = kflags; prm.knn_dub = dub; prm.knn_entries = entries;
-  prm.dbg_scores = nullptr;
   prm.neg_mu_s = nullptr; prm.assign = prm.prev = prm.d_changed = nullptr;
   prm.yy_qgroup = prm.yy_groups = prm.yy_assign = nullptr; prm.yy_bounds = nullptr; prm.G = 0;
   prm.knn_part = part; prm.knn_nparts = nparts ? nparts : 1;

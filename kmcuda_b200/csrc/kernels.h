@@ -45,10 +45,7 @@ struct UpdateWorkspace {
   size_t cub_tmp_bytes = 0;
   uint32_t iota_n = 0;           // vals_in[0 .. iota_n) already holds the identity permutation
 };
-#ifndef KMB_SUM_CHUNK
-#define KMB_SUM_CHUNK 512
-#endif
-constexpr uint32_t kSumChunk = KMB_SUM_CHUNK;   // sorted positions per CTA of the member-sum kernel
+constexpr uint32_t kSumChunk = 512;   // sorted positions per CTA of the member-sum kernel
 size_t update_partial_rows(uint32_t n, uint32_t K);
 size_t update_cub_bytes(uint32_t n);
 // sums[K][D] (fp32) and counts[K] (uint32) of this shard's samples
@@ -200,8 +197,7 @@ uint32_t tc_last_error(TcPlan* plan);
 uint32_t tc_last_pairs(TcPlan* plan);
 void tc_set_capture(TcPlan* plan, bool on);   // the next tc_assign is recorded into a CUDA graph (stream capture)
 int tc_kernel_times(TcPlan* plan, float* ms_out, int max_out);
-// diagnostics (KMCUDA_B200_DUMP_SCORES=1): approximate scores [tiles*128][nt*256], prep statistics
-const float* tc_debug_scores(TcPlan* plan, size_t* row_stride);
+// diagnostics: prep statistics
 void tc_debug_stats(TcPlan* plan, float* out4);
 
 }  // namespace kmb

@@ -396,15 +396,6 @@ uint32_t kmcuda_b200_debug_last_error(kmcuda_b200_shard* shard) {
   if (!shard || !shard->impl->tc) return 0;
   return kmb::tc_last_error(shard->impl->tc);
 }
-// copies rows x cols of the dumped approximate scores (KMCUDA_B200_DUMP_SCORES=1) to host memory
-int32_t kmcuda_b200_debug_scores(kmcuda_b200_shard* shard, float* host_out, uint32_t rows, uint32_t cols) {
-  if (!shard || !shard->impl->tc) return -1;
-  size_t stride = 0;
-  const float* src = kmb::tc_debug_scores(shard->impl->tc, &stride);
-  if (!src || cols > stride) return -2;
-  return cudaMemcpy2D(host_out, cols * sizeof(float), src, stride * sizeof(float), cols * sizeof(float), rows,
-                      cudaMemcpyDeviceToHost) == cudaSuccess ? 0 : -3;
-}
 // device time (ms) of the tensor-core kernel in the most recent passes (CUDA events on the launching
 // stream), oldest first; returns how many were written.  Call after synchronising the stream.
 int32_t kmcuda_b200_kernel_times(kmcuda_b200_shard* shard, float* ms_out, int32_t max_out) {

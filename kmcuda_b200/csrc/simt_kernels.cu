@@ -384,20 +384,7 @@ static void launch_segment_offsets(const uint32_t* keys, uint32_t n, uint32_t K,
   segment_offsets_kernel<<<cdiv((static_cast<size_t>(K) + 1) * 32, 128), 128, 0, st>>>(keys, n, K, offsets, counts);
 }
 
-#ifndef KMB_UPDATE_UNROLL
-#define KMB_UPDATE_UNROLL 8
-#endif
-constexpr int kUpdateUnroll = KMB_UPDATE_UNROLL;
-#ifndef KMB_SUM_STREAMING
-#define KMB_SUM_STREAMING 1   // 1: ld.global.cs (evict-first) for the sample rows, which are read once
-#endif
-__device__ __forceinline__ float sum_load(const float* p) {
-#if KMB_SUM_STREAMING
-  return __ldcs(p);
-#else
-  return __ldg(p);
-#endif
-}
+constexpr int kUpdateUnroll = 8;
 
 // Member sums, balanced: CTA b owns the sorted positions [b * kSumChunk, (b + 1) * kSumChunk) whatever clusters they
 // belong to, and writes one partial row per (chunk, cluster) run it meets, into slot b + c (unique: along the sorted
@@ -405,7 +392,8 @@ __device__ __forceinline__ float sum_load(const float* p) {
 // per cluster -- made the pass as slow as the largest cluster (4.9 ms instead of 2.1 ms at 8M x 256 @ 1024 when the
 // centroids are random rows and the cell sizes differ by an order of magnitude).  Within a run the additions are
 // compensated and in sample order, kUpdateUnroll member rows in flight per thread (with 4 the gather ran at
-// ~4.7 TB/s, short of the bytes in flight the HBM latency asks for).
+// ~4.7 TB/s, short of the bytes in flight the HBM latency asks for).  The sample rows are read once, so they are loaded
+// with ld.global.cs (evict-first).
 // (VEC = 4: D % 4 == 0 and 16-byte aligned rows -- a thread owns four adjacent features and reads them with one
 // 16-byte load, so a CTA is D / 4 threads and every thread keeps 8 x 16 bytes in flight: the gather is latency-bound,
 // 2.26 ms at 8M x 256 with 4-byte loads and 8 rows in flight, 1.89 ms with 16 rows in flight)
@@ -438,14 +426,10 @@ cluster_sums_kernel(const float* __restrict__ X, int D, const uint32_t* __restri
         for (int u = 0; u < kUpdateUnroll; u++) {
           const float* src = X + static_cast<size_t>(id[u]) * D + f * VEC;
           if (VEC == 4) {
-#if KMB_SUM_STREAMING
             const float4 t4 = __ldcs(reinterpret_cast<const float4*>(src));
-#else
-            const float4 t4 = __ldg(reinterpret_cast<const float4*>(src));
-#endif
             v[u][0] = t4.x; v[u][VEC > 1 ? 1 : 0] = t4.y; v[u][VEC > 2 ? 2 : 0] = t4.z; v[u][VEC > 3 ? 3 : 0] = t4.w;
           } else {
-            v[u][0] = sum_load(src);
+            v[u][0] = __ldcs(src);
           }
         }
 #pragma unroll
@@ -463,7 +447,7 @@ cluster_sums_kernel(const float* __restrict__ X, int D, const uint32_t* __restri
         const float* src = X + static_cast<size_t>(idx[j]) * D + f * VEC;
 #pragma unroll
         for (int q = 0; q < VEC; q++) {
-          const float y = sum_load(src + q) - comp[q], t = sum[q] + y;
+          const float y = __ldcs(src + q) - comp[q], t = sum[q] + y;
           comp[q] = (t - sum[q]) - y;
           sum[q] = t;
         }

@@ -45,6 +45,8 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t by
 // spun without a hint: 14 SASS instructions per probe and ~40 % of all issued instructions of the kernel were
 // such probes (profiles/r01_tc_assign_v4: 150 M SYNCS + 350 M BRA), stolen from the converter / epilogue warps
 // of the same scheduler.
+constexpr uint32_t kWaitHintNs = 2000;    // inline probe of every wait
+constexpr uint32_t kSlowHintNs = 20000;   // probes of the out-of-line remainder (mbar_wait_slow)
 __device__ __forceinline__ bool mbar_try_wait(uint32_t addr, uint32_t parity, uint32_t hint_ns) {
   uint32_t done;
   asm volatile(
@@ -56,28 +58,11 @@ __device__ __forceinline__ bool mbar_try_wait(uint32_t addr, uint32_t parity, ui
       : "memory");
   return done != 0;
 }
-#ifndef KMB_WAIT_HINT_NS
-#define KMB_WAIT_HINT_NS 2000   // 0 = A/B build: plain polling without a suspend hint
-#endif
-__device__ __forceinline__ bool mbar_try_wait_nohint(uint32_t addr, uint32_t parity) {
-  uint32_t done;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(done)
-      : "r"(addr), "r"(parity)
-      : "memory");
-  return done != 0;
-}
 // Out-of-line remainder of every wait: a TIGHT polling loop (round 2's first version re-checked the error word and
 // the clock in the loop body: ncu counted 0.9 G warp instructions per pass -- a third of everything the kernel issued --
 // in that loop, because a hinted try_wait returns on every update of the barrier, not only when the phase flips).
 // `site` names the waiting role; after ~2 s (or as soon as another thread has reported an error) the wait gives up and
 // reports 0x1000 + site in *err: a stuck pipeline must not hang the GPU box.
-#ifndef KMB_SLOW_HINT_NS
-#define KMB_SLOW_HINT_NS 20000
-#endif
 __device__ __noinline__ void mbar_wait_slow(uint32_t addr, uint32_t parity, uint32_t* err, uint32_t site, uint32_t flag_u32) {
   // flag_u32: a word of this CTA's shared memory that is set once any wait of the CTA has given up; from then on every
   // wait returns at once, so a broken pipeline drains in milliseconds instead of timing out wait by wait
@@ -92,11 +77,7 @@ __device__ __noinline__ void mbar_wait_slow(uint32_t addr, uint32_t parity, uint
         "{\n\t.reg .pred p, q;\n\t.reg .b32 c;\n\t"
         "mov.u32 c, 0;\n"
         "KMB_WAIT_LOOP_%=:\n\t"
-#if KMB_WAIT_HINT_NS > 0
         "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-#else
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-#endif
         "@p bra KMB_WAIT_DONE_%=;\n\t"
         "add.u32 c, c, 1;\n\t"
         "setp.lt.u32 q, c, 1024;\n\t"
@@ -104,7 +85,7 @@ __device__ __noinline__ void mbar_wait_slow(uint32_t addr, uint32_t parity, uint
         "KMB_WAIT_DONE_%=:\n\t"
         "selp.u32 %0, 1, 0, p;\n\t}"
         : "=r"(done)
-        : "r"(addr), "r"(parity), "r"(static_cast<uint32_t>(KMB_SLOW_HINT_NS))
+        : "r"(addr), "r"(parity), "r"(kSlowHintNs)
         : "memory");
     if (done) return;
     asm volatile("ld.volatile.shared.u32 %0, [%1];" : "=r"(dead) : "r"(flag_u32));
@@ -118,19 +99,7 @@ __device__ __noinline__ void mbar_wait_slow(uint32_t addr, uint32_t parity, uint
 }
 // The inline part: one probe (with the suspend hint it may sleep up to the hint while the phase has not flipped).
 __device__ __forceinline__ void mbar_wait(uint32_t addr, uint32_t parity, uint32_t* err, uint32_t site, uint32_t flag_u32) {
-#if KMB_WAIT_HINT_NS > 0
-  if (!mbar_try_wait(addr, parity, KMB_WAIT_HINT_NS)) mbar_wait_slow(addr, parity, err, site, flag_u32);
-#else
-  if (!mbar_try_wait_nohint(addr, parity)) mbar_wait_slow(addr, parity, err, site, flag_u32);
-#endif
-}
-// The MMA issuer's wait: plain polling first (no suspend: the issuer is the one warp whose wake-up latency is paid by
-// the tensor pipe).
-__device__ __forceinline__ void mbar_wait_spin(uint32_t addr, uint32_t parity, uint32_t* err, uint32_t site, uint32_t flag_u32) {
-#pragma unroll 1
-  for (int i = 0; i < 64; i++)
-    if (mbar_try_wait_nohint(addr, parity)) return;
-  mbar_wait_slow(addr, parity, err, site, flag_u32);
+  if (!mbar_try_wait(addr, parity, kWaitHintNs)) mbar_wait_slow(addr, parity, err, site, flag_u32);
 }
 
 // ---------------------------------------------------------------------------- packed fp32 pairs (sm_100: FADD2 / FMUL2 / FFMA2)

@@ -32,8 +32,6 @@ _lib.kmcuda_b200_kernel_times.restype = ctypes.c_int32
 _lib.kmcuda_b200_kernel_times.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32]
 _lib.kmcuda_b200_debug_last_error.restype = ctypes.c_uint32
 _lib.kmcuda_b200_debug_last_error.argtypes = [ctypes.c_void_p]
-_lib.kmcuda_b200_debug_scores.restype = ctypes.c_int32
-_lib.kmcuda_b200_debug_scores.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32, ctypes.c_uint32]
 _lib.kmcuda_b200_debug_yy_bounds.restype = ctypes.c_int32
 _lib.kmcuda_b200_debug_yy_bounds.argtypes = [ctypes.c_void_p, ctypes.c_uint32, ctypes.c_void_p, ctypes.c_void_p,
                                              ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32, ctypes.c_int32,
@@ -136,13 +134,6 @@ class Shard:
                                                   _stream_ptr()), "kmcuda_b200_finish_update")
 
     # diagnostics
-    def debug_scores(self, rows, cols):
-        out = np.empty((rows, cols), np.float32)
-        rc = _lib.kmcuda_b200_debug_scores(self._h, out.ctypes.data, rows, cols)
-        if rc != 0:
-            raise RuntimeError("debug scores unavailable (%d); set KMCUDA_B200_DUMP_SCORES=1" % rc)
-        return out
-
     def debug_yy_bounds(self, X, C, assignments, groups, G, use_tc):
         """Yinyang bounds [n][G + 1] of one refresh (diagnostics / parity tests); groups: host uint32 [K]"""
         groups = np.ascontiguousarray(groups, dtype=np.uint32)

@@ -1,4 +1,4 @@
-# A/B timing of kernel variants (variants/<name>/libKMCUDA.so, built with kmcuda_b200/build.py --variant);
+# A/B timing of other builds of the library (variants/<name>/libKMCUDA.so, e.g. built at another commit);
 # optional: "ncu" = one ncu --set full capture of the product kernel, "tests" = the GPU test suite
 mkdir -p gpurun_out
 export PATH=/usr/local/cuda/bin:$PATH

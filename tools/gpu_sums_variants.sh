@@ -1,4 +1,4 @@
-# member-sum variants (chunk size, streaming loads, unroll) at 8M and 1M rows
+# the member-sum pass of the product build and of every variants/*/libKMCUDA.so at 8M and 1M rows
 mkdir -p gpurun_out
 export PATH=/usr/local/cuda/bin:$PATH
 for n in 8000000 1000000; do
